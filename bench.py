@@ -20,6 +20,10 @@ Workloads (BASELINE.json configs):
           all-reduced into the reference's pair order, host graph on every rank.  torch.distributed only hands the NCCL id
           around and provides the barrier / max-over-ranks.  Same workload at every N => "scaling": "strong".
   --impl reference : the CPU restatement of the reference (oracle/, all host threads), bounded sample per step.
+
+  --dump-outputs DIR : after the timed steps, what the last timed step returned to its caller is saved as DIR/<name>.npy
+          (transforms.npy, or composed_points.npy for c5), at most 64 MB in all; the inputs are seeded, so two builds run
+          with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -33,11 +37,21 @@ import time
 
 import numpy as np
 
+# the benchmark runs from the tree as built and writes nothing into it (the tree may be read-only)
+sys.dont_write_bytecode = True
+
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 METRIC = "pairwise_registrations_per_sec"
 UNIT = "pairs/s"
+
+# roofline denominator: HBM copy bandwidth (read + write) measured on an NVIDIA B200 at SM max 1965 MHz, power limit not
+# recorded (BASELINE.md section 2)
+HBM_PEAK_GBS = 6453.7
+HBM_PEAK_SOURCE = "HBM copy bandwidth measured on a B200 (BASELINE.md section 2)"
+
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this many bytes of files in all
 
 WORKLOADS = {
     "c2": dict(params=dict(descriptor_type="FPFH"), what="SIFT+FPFH, MATCHING+ICP"),
@@ -63,12 +77,19 @@ def workload_label(name, cfg):
     return f"{name}: {m} maps x {cfg['n_points']} pts, {WORKLOADS[name]['what']}, {n_pairs_of(m)} pairs"
 
 
-def measured_peak():
-    try:
-        with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
-            return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
-    except Exception:
-        return 6650.0, "fallback (B200_PROFILING.md)"
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Saves every array as <out_dir>/<name>.npy, the files ``budget`` bytes at most in all.  An array larger than its share
+    is cut to a fixed, seeded sample of its rows, kept in their original order, so that the files of two runs line up row
+    for row."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = budget // len(arrays) - 4096  # room for the .npy header
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        if a.nbytes > share:
+            rows = share // (a.nbytes // len(a))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), rows, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -187,10 +208,12 @@ def run_reference(args):
     t_run = time.perf_counter()
     done = 0
     for s in range(total_steps):
-        f, g, _ = oracle_sample_job(O, sub, p)
+        f, g, r = oracle_sample_job(O, sub, p)
         done += 1
         if s >= args.warmup:
             feats.append(f); pairs.append(g)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"transforms": r["transforms"]})
     full = M * float(np.mean(feats)) + P * float(np.mean(pairs))
     value = P / full
     line = {
@@ -223,9 +246,11 @@ def run_reference_compose(args):
     times = []
     for s in range(args.steps + args.warmup):
         t0 = time.perf_counter()
-        O.compose_maps(maps[:1], T, 0.05)
+        out = O.compose_maps(maps[:1], T, 0.05)
         if s >= args.warmup:
             times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"composed_points": out})
     per_map = float(np.mean(times))
     value = cfg["n_points"] / per_map
     line = {"impl": "reference", "metric": "compose_maps_points_per_sec", "value": value, "unit": "points/s", "n_gpus": args.gpus,
@@ -464,10 +489,11 @@ def run_gpu(args):
     _, _, prof, _, _ = job.timed(psteps, lambda: job.step(False), profile=True)
     if job.rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"transforms": out})  # every rank holds all transforms
     value = P * args.steps / (ms * 1e-3)
     e2e = P * args.steps / (ms_e2e * 1e-3)
-    peak, peak_src = measured_peak()
-    roof, kernels = roofline_of(prof, psteps, peak, peak_src)
+    roof, kernels = roofline_of(prof, psteps, HBM_PEAK_GBS, HBM_PEAK_SOURCE)
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": job.world, "steps": args.steps, "warmup": W,
         "ms_per_step": ms / args.steps, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -518,10 +544,14 @@ def run_gpu_compose(args, job):
     n_out = job.torch.tensor([len(out)], dtype=job.torch.int64, device=job.dev)
     if job.world > 1:
         job.dist.all_reduce(n_out)
+    if args.dump_outputs:
+        # each rank returns its own key range of the composed map
+        name = "composed_points" if job.world == 1 else f"composed_points_rank{job.rank}"
+        dump_outputs(args.dump_outputs, {name: out}, DUMP_BYTES // job.world)
     if job.rank != 0:
         return
-    peak, peak_src = measured_peak()
-    roof, kernels = roofline_of(prof, psteps, peak, peak_src)
+    peak = HBM_PEAK_GBS
+    roof, kernels = roofline_of(prof, psteps, peak, HBM_PEAK_SOURCE)
     # whole-step roofline: every input point read once, transformed copy written and read once, output written once
     step_bytes = 48.0 * n_in / job.world + 16.0 * len(out)
     kernel_ms = sum(k["ms"] for k in prof) / psteps
@@ -557,7 +587,10 @@ def main():
     ap.add_argument("--impl", default="mm3d", choices=["mm3d", "reference"])
     ap.add_argument("--workload", default="c3", choices=sorted(set(WORKLOADS) | {"c5"}))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="save what the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     # stdout carries exactly one JSON line: keep a private handle to it and point fd 1 at stderr, so that anything a
     # library writes to stdout (NCCL prints its version banner there) cannot get in front of the line
     global _OUT
