@@ -92,6 +92,35 @@ int mm3d_estimate_maps_transforms(mm3d_ctx* ctx, int n_maps, const float* const*
 int mm3d_compose_maps(mm3d_ctx* ctx, int n_maps, const float* const* clouds, const uint64_t* n_points, int n_transforms,
                       const float* transforms, double resolution, float** out, uint64_t* n_out);
 
+/* ---- the high-level calls on points in the caller's own record layout ------------------------------------------------
+ * The records are converted to (and for outputs from) the packed layout on the GPU, so a caller that holds, for example,
+ * a std::vector<pcl::PointXYZRGB> hands it over as it is.  Input in the packed layout {16, 0, 4, 8, 12, NULL} is copied
+ * straight from the caller's buffer; any other layout goes through pinned staging slots of the context (host threads copy
+ * the records in, the device converts them).  Fields move as 32-bit words, so NaN payloads, infinities and -0.0 arrive
+ * bit for bit. */
+
+/* Where the fields of one point sit in a caller's array of records.  All offsets and point_step are byte counts and
+ * multiples of 4; each field is 4 bytes (float32 x, y, z; the 32-bit rgba word) and lies inside the record. */
+typedef struct mm3d_layout {
+  uint32_t point_step;                 /* bytes from one point to the next (16 = the packed layout, 32 = pcl::PointXYZRGB) */
+  int32_t offset_x, offset_y, offset_z, offset_rgba;
+  const void* record_template;         /* outputs only: point_step bytes that every output record starts from; NULL = zeros */
+} mm3d_layout;
+/* A layout is malformed (MM3D_ERR_ARG, nothing launched) when it is NULL, point_step < 16, point_step > MM3D_LAYOUT_MAX_STEP
+ * or not a multiple of 4, or an offset is negative, not a multiple of 4 or puts its field past the end of the record. */
+#define MM3D_LAYOUT_MAX_STEP 65536
+
+/* mm3d_estimate_maps_transforms on records in `layout` */
+int mm3d_estimate_maps_transforms_layout(mm3d_ctx* ctx, int n_maps, const void* const* clouds, const uint64_t* n_points,
+                                         const mm3d_layout* layout, const mm3d_params* params, float* out_transforms, int* n_out);
+/* mm3d_compose_maps on records in `in_layout`; *out = n_out records in `out_layout` (mm3d_free) */
+int mm3d_compose_maps_layout(mm3d_ctx* ctx, int n_maps, const void* const* clouds, const uint64_t* n_points, const mm3d_layout* in_layout,
+                             int n_transforms, const float* transforms, double resolution, const mm3d_layout* out_layout, void** out,
+                             uint64_t* n_out);
+/* mm3d_maps_upload on records in `layout` */
+int mm3d_maps_upload_layout(mm3d_ctx* ctx, int n_maps, const void* const* clouds, const uint64_t* n_points, const mm3d_layout* layout,
+                            mm3d_maps** maps);
+
 /* ---- low-level interface (features.h / matching.h) ------------------------ */
 /* index_leaf: voxel size the cloud was built with (MapMergingParams::resolution); 0 picks
  * radius / 8 (descriptor-style radii) or radius / 6 (normal-style radii), the reference's
@@ -153,7 +182,7 @@ int mm3d_global_transforms(int n_pairs, const int32_t* st, const float* transfor
 
 /* ---- resident interface (inputs already in HBM; what bench.py and the multi-GPU driver use) -- */
 
-/* Copies the clouds to the device once. */
+/* Copies the clouds to the device once (mm3d_maps_upload_layout takes other record layouts). */
 int mm3d_maps_upload(mm3d_ctx* ctx, int n_maps, const float* const* clouds, const uint64_t* n_points, mm3d_maps** maps);
 void mm3d_maps_free(mm3d_maps* maps);
 

@@ -44,7 +44,7 @@ SYMBOLS = [
     "mm3d_compose_shard_histogram", "mm3d_compose_shard_partition", "mm3d_compose_shard_points", "mm3d_shard_free", "mm3d_downsample_dev",
     "mm3d_knn", "mm3d_knn_tc_audit", "mm3d_create_multi", "mm3d_device_count", "mm3d_comm_id", "mm3d_comm_create", "mm3d_comm_destroy", "mm3d_comm_rank", "mm3d_comm_size",
     "mm3d_dist_block", "mm3d_dist_plan", "mm3d_estimate_maps_transforms_dist", "mm3d_estimate_resident_dist", "mm3d_compose_maps_dist",
-    "mm3d_compose_resident_dist",
+    "mm3d_compose_resident_dist", "mm3d_estimate_maps_transforms_layout", "mm3d_compose_maps_layout", "mm3d_maps_upload_layout",
 ]
 COMM_ID_BYTES = 128
 
@@ -59,6 +59,29 @@ class Params(C.Structure):
         ("matching_k", C.c_uint64), ("transform_epsilon", C.c_double), ("confidence_threshold", C.c_double),
         ("output_resolution", C.c_double),
     ]
+
+
+class Layout(C.Structure):
+    """mm3d_layout: byte offsets of x, y, z and rgba inside records of point_step bytes (include/mm3d.h).  record_template
+    (outputs only): point_step bytes every output record starts from, or None for zeros."""
+    _fields_ = [("point_step", C.c_uint32), ("offset_x", C.c_int32), ("offset_y", C.c_int32), ("offset_z", C.c_int32),
+                ("offset_rgba", C.c_int32), ("record_template", C.c_void_p)]
+
+    def __init__(self, point_step, offset_x, offset_y, offset_z, offset_rgba, record_template=None):
+        super().__init__(point_step, offset_x, offset_y, offset_z, offset_rgba, None)
+        if record_template is not None:
+            self._template = (C.c_uint8 * len(record_template)).from_buffer_copy(bytes(record_template))  # kept alive with the layout
+            self.record_template = C.addressof(self._template)
+
+    @property
+    def template_bytes(self) -> bytes:
+        return bytes(self._template) if self.record_template else bytes(self.point_step)
+
+
+PACKED = Layout(16, 0, 4, 8, 12)
+# pcl::PointXYZRGB: x y z, data[3] = 1.0f, rgba, three padding floats; a default-constructed point is (0, 0, 0, 1) with a = 255
+PCL_XYZRGB = Layout(32, 0, 4, 8, 16, np.array([0.0, 0.0, 0.0, 1.0], np.float32).tobytes() +
+                    np.array([0xff000000, 0, 0, 0], np.uint32).tobytes())
 
 
 class MM3DError(RuntimeError):
@@ -323,6 +346,49 @@ class Context:
         ptrs = (f32p * max(m, 1))(*[(a.ctypes.data_as(f32p) if a is not None and len(a) else f32p()) for a in arrs])
         ns = (C.c_uint64 * max(m, 1))(*[(len(a) if a is not None else 0) for a in arrs])
         return arrs, ptrs, ns
+
+    @staticmethod
+    def _record_args(clouds, layout: Layout):
+        """clouds: C-contiguous uint8 arrays of shape (n, layout.point_step), or None for an empty map."""
+        m = len(clouds)
+        arrs = []
+        for c in clouds:
+            if c is not None:
+                c = np.asarray(c)
+                if c.dtype != np.uint8 or c.ndim != 2 or c.shape[1] != layout.point_step or not c.flags.c_contiguous:
+                    raise ValueError(f"records must be a C-contiguous uint8 array of shape (n, {layout.point_step}), got {c.dtype} {c.shape}")
+            arrs.append(c)
+        ptrs = (C.c_void_p * max(m, 1))(*[(a.ctypes.data if a is not None and len(a) else None) for a in arrs])
+        ns = (C.c_uint64 * max(m, 1))(*[(len(a) if a is not None else 0) for a in arrs])
+        return arrs, ptrs, ns
+
+    def estimate_maps_transforms_layout(self, clouds, layout: Layout, params: Params):
+        """estimate_maps_transforms on records in `layout` (converted on the GPU)."""
+        arrs, ptrs, ns = self._record_args(clouds, layout)
+        m = len(clouds)
+        out = np.zeros((max(m, 1), 16), np.float32); no = C.c_int()
+        self._check(self.L.mm3d_estimate_maps_transforms_layout(self.h, m, ptrs, ns, C.byref(layout), C.byref(params), out.ctypes.data_as(f32p),
+                                                                C.byref(no)))
+        return out[:no.value].reshape(-1, 4, 4).transpose(0, 2, 1).copy()
+
+    def compose_maps_layout(self, clouds, transforms, resolution, in_layout: Layout, out_layout: Layout):
+        """compose_maps on records in `in_layout`; returns uint8[n, out_layout.point_step] records (None for no maps)."""
+        arrs, ptrs, ns = self._record_args(clouds, in_layout)
+        T = np.asarray(transforms, np.float32).reshape(-1, 4, 4)
+        Tc = np.ascontiguousarray(T.transpose(0, 2, 1)) if len(T) else np.zeros((1, 16), np.float32)
+        out = C.c_void_p(); n = C.c_uint64()
+        rc = self.L.mm3d_compose_maps_layout(self.h, len(clouds), ptrs, ns, C.byref(in_layout), len(T), Tc.ctypes.data_as(f32p),
+                                             C.c_double(resolution), C.byref(out_layout), C.byref(out), C.byref(n))
+        if rc == 1:
+            return None
+        self._check(rc)
+        return self._take(out, n.value * out_layout.point_step, np.uint8, (-1, out_layout.point_step))
+
+    def maps_upload_layout(self, clouds, layout: Layout):
+        arrs, ptrs, ns = self._record_args(clouds, layout)
+        h = C.c_void_p()
+        self._check(self.L.mm3d_maps_upload_layout(self.h, len(clouds), ptrs, ns, C.byref(layout), C.byref(h)))
+        return Maps(self, h, len(clouds))
 
     def estimate_maps_transforms(self, clouds, params: Params):
         arrs, ptrs, ns = self._cloud_args(clouds)

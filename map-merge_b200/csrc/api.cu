@@ -180,15 +180,6 @@ void from_colmajor(const float* cm, float* rm)
     for (int c = 0; c < 4; ++c) rm[r * 4 + c] = cm[c * 4 + r];
 }
 
-DCloud upload_cloud(Ctx& c, const float* pts, uint64_t n)
-{
-  DCloud d;
-  d.n = (pts ? (int)n : 0);
-  d.pts.alloc(c, d.n);
-  if (d.n) MM_CUDA(cudaMemcpyAsync(d.pts.p, pts, (size_t)d.n * sizeof(float4), cudaMemcpyHostToDevice, c.stream));
-  return d;
-}
-
 // src/map_merging.cpp:212-242, stage-major over all maps
 void compute_features(Ctx& c, const std::vector<CloudView>& raw, const mm3d_params& p, std::vector<MapFeat>& out, float* stage_ms)
 {
@@ -417,6 +408,12 @@ int estimate_from_views(Ctx& c, const std::vector<CloudView>& raw, const mm3d_pa
   return (int)g.size();
 }
 
+int bad_layout(mm3d_ctx* ctx)
+{
+  if (ctx) ctx->c.err = "malformed mm3d_layout (include/mm3d.h)";
+  return MM3D_ERR_ARG;
+}
+
 }  // namespace
 
 #define MM_TRY(ctx) \
@@ -500,6 +497,7 @@ void mm3d_destroy(mm3d_ctx* ctx)
   ctx->c.cache->trim();        // cached blocks go back while the stream still exists
   ctx->c.cache->stream = nullptr;  // blocks returned by buffers that outlive the context are freed with the last reference
   if (ctx->c.knn_stats) cudaFree(ctx->c.knn_stats);
+  staging_release(ctx->c);
   for (cudaEvent_t e : ctx->c.event_pool) cudaEventDestroy(e);
   for (KernelSample& s : ctx->c.samples) { cudaEventDestroy(s.e0); cudaEventDestroy(s.e1); }
   if (ctx->c.own_stream) cudaStreamDestroy(ctx->c.stream);
@@ -513,8 +511,15 @@ long long mm3d_kernel_launches(mm3d_ctx* ctx) { return ctx ? ctx->c.launches : 0
 int mm3d_estimate_maps_transforms(mm3d_ctx* ctx, int n_maps, const float* const* clouds, const uint64_t* n_points, const mm3d_params* params,
                                   float* out_transforms, int* n_out)
 {
+  return mm3d_estimate_maps_transforms_layout(ctx, n_maps, (const void* const*)clouds, n_points, &kPackedLayout, params, out_transforms, n_out);
+}
+
+int mm3d_estimate_maps_transforms_layout(mm3d_ctx* ctx, int n_maps, const void* const* clouds, const uint64_t* n_points,
+                                         const mm3d_layout* layout, const mm3d_params* params, float* out_transforms, int* n_out)
+{
   if (!n_out) return MM3D_ERR_ARG;
   *n_out = 0;
+  if (!layout_valid(layout)) return bad_layout(ctx);
   // the degenerate cases never touch the device (map_merging.cpp:192-197)
   if (n_maps == 0) return MM3D_OK;
   if (n_maps == 1) {
@@ -525,15 +530,12 @@ int mm3d_estimate_maps_transforms(mm3d_ctx* ctx, int n_maps, const float* const*
   }
   MM_TRY(ctx)
   if (ctx->team) {  // mm3d_create_multi: maps and pairs sharded over the context's devices (dist.cu)
-    *n_out = team_estimate(ctx, n_maps, clouds, n_points, *params, out_transforms);
+    *n_out = team_estimate(ctx, n_maps, clouds, n_points, *layout, *params, out_transforms);
     return MM3D_OK;
   }
-  std::vector<DCloud> d(n_maps);
+  std::vector<DCloud> d = upload_clouds(c, std::vector<const void*>(clouds, clouds + n_maps), std::vector<uint64_t>(n_points, n_points + n_maps), *layout);
   std::vector<CloudView> v(n_maps);
-  for (int m = 0; m < n_maps; ++m) {
-    d[m] = upload_cloud(c, clouds[m], clouds[m] ? n_points[m] : 0);
-    v[m] = d[m].view();
-  }
+  for (int m = 0; m < n_maps; ++m) v[m] = d[m].view();
   *n_out = estimate_from_views(c, v, *params, out_transforms, nullptr);
   c.sync();
   MM_CATCH
@@ -542,9 +544,18 @@ int mm3d_estimate_maps_transforms(mm3d_ctx* ctx, int n_maps, const float* const*
 int mm3d_compose_maps(mm3d_ctx* ctx, int n_maps, const float* const* clouds, const uint64_t* n_points, int n_transforms,
                       const float* transforms, double resolution, float** out, uint64_t* n_out)
 {
+  return mm3d_compose_maps_layout(ctx, n_maps, (const void* const*)clouds, n_points, &kPackedLayout, n_transforms, transforms, resolution,
+                                  &kPackedLayout, (void**)out, n_out);
+}
+
+int mm3d_compose_maps_layout(mm3d_ctx* ctx, int n_maps, const void* const* clouds, const uint64_t* n_points, const mm3d_layout* in_layout,
+                             int n_transforms, const float* transforms, double resolution, const mm3d_layout* out_layout, void** out,
+                             uint64_t* n_out)
+{
   if (!out || !n_out) return MM3D_ERR_ARG;
   *out = nullptr;
   *n_out = 0;
+  if (!layout_valid(in_layout) || !layout_valid(out_layout)) return bad_layout(ctx);
   if (n_maps == 0) return 1;  // nullptr result
   if (n_maps != n_transforms) {
     if (ctx) ctx->c.err = "composeMaps: clouds and transforms size must be the same.";
@@ -555,16 +566,16 @@ int mm3d_compose_maps(mm3d_ctx* ctx, int n_maps, const float* const* clouds, con
   for (int m = 0; m < n_maps; ++m)
     if (clouds[m] && n_points[m] > 0) any = true;
   if (!any) {
-    *out = (float*)malloc(16);
+    *out = malloc(16);
     return MM3D_OK;
   }
   MM_TRY(ctx)
   if (ctx->team) {
-    team_compose(ctx, n_maps, clouds, n_points, transforms, resolution, out, n_out);
+    team_compose(ctx, n_maps, clouds, n_points, *in_layout, transforms, resolution, *out_layout, out, n_out);
     return MM3D_OK;
   }
-  std::vector<DCloud> d;
-  std::vector<CloudView> v;
+  std::vector<const void*> src;
+  std::vector<uint64_t> cnt;
   std::vector<std::vector<float>> tr;
   for (int m = 0; m < n_maps; ++m) {
     float rm[16];
@@ -573,9 +584,12 @@ int mm3d_compose_maps(mm3d_ctx* ctx, int n_maps, const float* const* clouds, con
     for (int k = 0; k < 16; ++k)
       if (!(std::fabs(rm[k]) <= 1e-5f)) zero = false;
     if (zero || !clouds[m] || n_points[m] == 0) continue;
-    d.push_back(upload_cloud(c, clouds[m], n_points[m]));
+    src.push_back(clouds[m]);
+    cnt.push_back(n_points[m]);
     tr.emplace_back(rm, rm + 16);
   }
+  std::vector<DCloud> d = upload_clouds(c, src, cnt, *in_layout);
+  std::vector<CloudView> v;
   std::vector<const float*> tp;
   for (size_t i = 0; i < d.size(); ++i) {
     v.push_back(d[i].view());
@@ -585,7 +599,7 @@ int mm3d_compose_maps(mm3d_ctx* ctx, int n_maps, const float* const* clouds, con
   transform_concat(c, v, tp, cat);
   std::vector<DCloud> res;
   voxel_downsample_batch(c, {cat.view()}, (float)resolution, res, nullptr);
-  *out = (float*)host_copy(c, res[0].pts.p, (size_t)res[0].n);
+  *out = download_records(c, res[0].pts.p, (size_t)res[0].n, *out_layout);
   *n_out = (uint64_t)res[0].n;
   c.sync();
   MM_CATCH
@@ -1064,12 +1078,18 @@ int mm3d_downsample_dev(mm3d_ctx* ctx, const void* points_dev, uint64_t n, doubl
 
 int mm3d_maps_upload(mm3d_ctx* ctx, int n_maps, const float* const* clouds, const uint64_t* n_points, mm3d_maps** maps)
 {
+  return mm3d_maps_upload_layout(ctx, n_maps, (const void* const*)clouds, n_points, &kPackedLayout, maps);
+}
+
+int mm3d_maps_upload_layout(mm3d_ctx* ctx, int n_maps, const void* const* clouds, const uint64_t* n_points, const mm3d_layout* layout,
+                            mm3d_maps** maps)
+{
   if (!maps) return MM3D_ERR_ARG;
   *maps = nullptr;
+  if (!layout_valid(layout)) return bad_layout(ctx);
   MM_TRY(ctx)
   std::unique_ptr<mm3d_maps> h(new mm3d_maps);
-  h->clouds.resize(n_maps);
-  for (int m = 0; m < n_maps; ++m) h->clouds[m] = upload_cloud(c, clouds[m], clouds[m] ? n_points[m] : 0);
+  h->clouds = upload_clouds(c, std::vector<const void*>(clouds, clouds + n_maps), std::vector<uint64_t>(n_points, n_points + n_maps), *layout);
   c.sync();
   *maps = h.release();
   MM_CATCH

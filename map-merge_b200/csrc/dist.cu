@@ -365,9 +365,9 @@ std::vector<int> choose_splitters(const std::vector<unsigned long long>& hist, i
 }
 
 // One rank's part of composeMaps: local clouds already on the device.  Returns this rank's slice of the composed map on the
-// host (malloc); the slices concatenated in rank order are the reference's output bit for bit.
+// host (host_out_alloc, records in out_layout); the slices concatenated in rank order are the reference's output bit for bit.
 void dist_compose(Ctx& c, mm3d_comm* cm, const std::vector<CloudView>& local, const std::vector<const float*>& transforms_rowmajor,
-                  double resolution, float** out, uint64_t* n_out)
+                  double resolution, const mm3d_layout& out_layout, void** out, uint64_t* n_out)
 {
   const int W = cm ? cm->world : 1;
   constexpr int NB = 4096;
@@ -405,8 +405,7 @@ void dist_compose(Ctx& c, mm3d_comm* cm, const std::vector<CloudView>& local, co
     for (int k = 0; k < 3; ++k) { bbox[k] = h[k]; bbox[3 + k] = -h[3 + k]; }
   }
   auto to_host = [&](const float4* p, size_t n) {
-    *out = (float*)host_out_alloc(std::max<size_t>(n, 1) * 16);
-    if (n) MM_CUDA(cudaMemcpyAsync(*out, p, n * 16, cudaMemcpyDeviceToHost, c.stream));
+    *out = download_records(c, p, n, out_layout);
     *n_out = n;
     c.sync();
     mark("copy to the host");
@@ -469,7 +468,7 @@ void dist_compose(Ctx& c, mm3d_comm* cm, const std::vector<CloudView>& local, co
 }
 
 // composeMaps' skip rules (map_merging.cpp:293-295): zero transforms and empty clouds are left out
-bool skip_map(const float* colmajor, const float* cloud, uint64_t n, float* rowmajor)
+bool skip_map(const float* colmajor, const void* cloud, uint64_t n, float* rowmajor)
 {
   from_colmajor(colmajor, rowmajor);
   bool zero = true;  // Eigen isZero(): every |a_ij| <= 1e-5
@@ -519,9 +518,9 @@ namespace mm3d {
 
 int team_size(const mm3d_ctx* ctx) { return ctx && ctx->team ? (int)ctx->team->comms.size() : 1; }
 
-// estimateMapsTransforms from host buffers over the devices of a mm3d_create_multi context
-int team_estimate(mm3d_ctx* master, int n_maps, const float* const* clouds, const uint64_t* n_points, const mm3d_params& p,
-                  float* out_transforms)
+// estimateMapsTransforms from host buffers over the devices of a mm3d_create_multi context; each device uploads its own block
+int team_estimate(mm3d_ctx* master, int n_maps, const void* const* clouds, const uint64_t* n_points, const mm3d_layout& layout,
+                  const mm3d_params& p, float* out_transforms)
 {
   int n_out = 0;
   const int W = team_size(master);
@@ -530,12 +529,10 @@ int team_estimate(mm3d_ctx* master, int n_maps, const float* const* clouds, cons
   team_run(master, [&](int r, Ctx& c, mm3d_comm* cm) {
     int first, count;
     block_of(r, W, n_maps, &first, &count);
-    std::vector<DCloud> d(count);
+    std::vector<DCloud> d = upload_clouds(c, std::vector<const void*>(clouds + first, clouds + first + count),
+                                          std::vector<uint64_t>(n_points + first, n_points + first + count), layout);
     std::vector<CloudView> v(count);
-    for (int m = 0; m < count; ++m) {
-      d[m] = upload_cloud(c, clouds[first + m], clouds[first + m] ? n_points[first + m] : 0);
-      v[m] = d[m].view();
-    }
+    for (int m = 0; m < count; ++m) v[m] = d[m].view();
     counts[r] = dist_estimate(c, cm, n_maps, v, p, outs[r].data(), nullptr);
     c.sync();
   });
@@ -545,42 +542,46 @@ int team_estimate(mm3d_ctx* master, int n_maps, const float* const* clouds, cons
 }
 
 // composeMaps from host buffers over the devices of a mm3d_create_multi context
-void team_compose(mm3d_ctx* master, int n_maps, const float* const* clouds, const uint64_t* n_points, const float* transforms,
-                  double resolution, float** out, uint64_t* n_out)
+void team_compose(mm3d_ctx* master, int n_maps, const void* const* clouds, const uint64_t* n_points, const mm3d_layout& in_layout,
+                  const float* transforms, double resolution, const mm3d_layout& out_layout, void** out, uint64_t* n_out)
 {
   const int W = team_size(master);
-  std::vector<float*> parts(W, nullptr);
+  std::vector<void*> parts(W, nullptr);
   std::vector<uint64_t> sizes(W, 0);
   try {
     team_run(master, [&](int r, Ctx& c, mm3d_comm* cm) {
       int first, count;
       block_of(r, W, n_maps, &first, &count);
-      std::vector<DCloud> d;
+      std::vector<const void*> src;
+      std::vector<uint64_t> cnt;
       std::vector<std::vector<float>> tr;
       for (int m = first; m < first + count; ++m) {
         float rm[16];
         if (skip_map(transforms + 16 * m, clouds[m], n_points[m], rm)) continue;
-        d.push_back(upload_cloud(c, clouds[m], n_points[m]));
+        src.push_back(clouds[m]);
+        cnt.push_back(n_points[m]);
         tr.emplace_back(rm, rm + 16);
       }
+      std::vector<DCloud> d = upload_clouds(c, src, cnt, in_layout);
       std::vector<CloudView> v;
       std::vector<const float*> tp;
       for (size_t i = 0; i < d.size(); ++i) {
         v.push_back(d[i].view());
         tp.push_back(tr[i].data());
       }
-      dist_compose(c, cm, v, tp, resolution, &parts[r], &sizes[r]);
+      dist_compose(c, cm, v, tp, resolution, out_layout, &parts[r], &sizes[r]);
     });
   } catch (...) {
-    for (float* p : parts) host_out_free(p);
+    for (void* p : parts) host_out_free(p);
     throw;
   }
+  const size_t step = out_layout.point_step;
   uint64_t total = 0;
   for (uint64_t s : sizes) total += s;
-  *out = (float*)host_out_alloc(std::max<uint64_t>(total, 1) * 16);
+  *out = host_out_alloc(std::max<uint64_t>(total, 1) * step);
   uint64_t o = 0;
   for (int r = 0; r < W; ++r) {
-    if (sizes[r]) memcpy(*out + o * 4, parts[r], sizes[r] * 16);
+    if (sizes[r]) memcpy((unsigned char*)*out + o * step, parts[r], sizes[r] * step);
     o += sizes[r];
     host_out_free(parts[r]);
   }
@@ -742,7 +743,7 @@ int mm3d_compose_maps_dist(mm3d_ctx* ctx, mm3d_comm* comm, int n_local, const fl
     v.push_back(d[i].view());
     tp.push_back(tr[i].data());
   }
-  dist_compose(c, comm, v, tp, resolution, out, n_out);
+  dist_compose(c, comm, v, tp, resolution, kPackedLayout, (void**)out, n_out);
   MMD_CATCH
 }
 
@@ -768,7 +769,7 @@ int mm3d_compose_resident_dist(mm3d_ctx* ctx, mm3d_comm* comm, const mm3d_maps* 
     tr.emplace_back(rm, rm + 16);
   }
   for (size_t i = 0; i < tr.size(); ++i) tp.push_back(tr[i].data());
-  dist_compose(c, comm, v, tp, resolution, out, n_out);
+  dist_compose(c, comm, v, tp, resolution, kPackedLayout, (void**)out, n_out);
   MMD_CATCH
 }
 

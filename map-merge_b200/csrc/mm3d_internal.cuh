@@ -133,6 +133,8 @@ struct BlockCache {
   }
 };
 
+struct StagingRing;  // layout.cu: pinned slots for records in a caller's layout
+
 struct Ctx {
   int device = 0;
   std::shared_ptr<BlockCache> cache = std::make_shared<BlockCache>();
@@ -145,6 +147,7 @@ struct Ctx {
   unsigned long long* knn_stats = nullptr;  // device: rows, rows that fell back to the exact scan, candidates re-ranked
   std::vector<KernelSample> samples;
   std::vector<cudaEvent_t> event_pool;
+  StagingRing* staging = nullptr;  // created by the first staged upload, freed by mm3d_destroy (staging_release)
   void sync()
   {
     HostProf& hp = host_prof();

@@ -54,14 +54,25 @@ int desc_dim(const mm3d_params& p);
 std::vector<FeatView> feat_views(const std::vector<MapFeat>& f);
 void to_colmajor(const float* rm, float* cm);
 void from_colmajor(const float* cm, float* rm);
-DCloud upload_cloud(Ctx& c, const float* pts, uint64_t n);
+
+// layout.cu: records in a caller's layout (include/mm3d.h, mm3d_layout)
+extern const mm3d_layout kPackedLayout;  // {16, 0, 4, 8, 12, NULL}
+bool layout_valid(const mm3d_layout* l);
+bool layout_packed(const mm3d_layout& l);
+// host records in layout l -> device clouds (a NULL pointer is an empty cloud); the copies are enqueued on c.stream and
+// the caller's buffers are no longer read when the call returns
+std::vector<DCloud> upload_clouds(Ctx& c, const std::vector<const void*>& src, const std::vector<uint64_t>& n, const mm3d_layout& l);
+DCloud upload_cloud(Ctx& c, const float* pts, uint64_t n);  // one cloud in the packed layout
+// n device points -> n records in layout l in a host_out_alloc block; the copy is enqueued on c.stream (the caller synchronises)
+void* download_records(Ctx& c, const float4* pts, size_t n, const mm3d_layout& l);
+void staging_release(Ctx& c);
 
 // dist.cu: the high-level calls over the devices of a mm3d_create_multi context (one host thread per device)
 int team_size(const mm3d_ctx* ctx);
-int team_estimate(mm3d_ctx* master, int n_maps, const float* const* clouds, const uint64_t* n_points, const mm3d_params& p,
-                  float* out_transforms);
-void team_compose(mm3d_ctx* master, int n_maps, const float* const* clouds, const uint64_t* n_points, const float* transforms,
-                  double resolution, float** out, uint64_t* n_out);
+int team_estimate(mm3d_ctx* master, int n_maps, const void* const* clouds, const uint64_t* n_points, const mm3d_layout& layout,
+                  const mm3d_params& p, float* out_transforms);
+void team_compose(mm3d_ctx* master, int n_maps, const void* const* clouds, const uint64_t* n_points, const mm3d_layout& in_layout,
+                  const float* transforms, double resolution, const mm3d_layout& out_layout, void** out, uint64_t* n_out);
 
 }  // namespace mm3d
 

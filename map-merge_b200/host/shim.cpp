@@ -2,8 +2,9 @@
 //
 // Function-for-function stand-in for the reference's static library `map_merging`
 // (map_merge_3d/CMakeLists.txt:67-74: features.cpp, matching.cpp, map_merging.cpp, graph.cpp).
-// Only data marshalling happens here: PCL's 32-byte points are packed to the 16-byte device layout,
-// errors become the exceptions / in-band sentinels the reference uses.  There is no CPU fallback.
+// Only data marshalling happens here: estimateMapsTransforms and composeMaps hand PCL's 32-byte points to the library as
+// they are (mm3d_layout; the GPU converts them), the low-level functions pack them to the 16-byte device layout, and errors
+// become the exceptions / in-band sentinels the reference uses.  There is no CPU fallback.
 #include <map_merge_3d/map_merging.h>
 
 #include <cstdlib>
@@ -88,6 +89,28 @@ PointCloudPtr unpack(const float* pts, uint64_t n)
   out->height = 1;
   out->is_dense = true;
   return out;
+}
+
+// Where x, y, z and rgba sit in a PointT, taken from a default-constructed point (PCL's PointXYZRGB is not standard-layout,
+// so offsetof does not apply); output records start as that point's bytes.
+const mm3d_layout& point_layout()
+{
+  static const PointT proto;
+  auto at = [](const void* field) { return (int32_t)((const char*)field - (const char*)&proto); };
+  static const mm3d_layout l = {(uint32_t)sizeof(PointT), at(&proto.x), at(&proto.y), at(&proto.z), at(&proto.rgba), &proto};
+  return l;
+}
+
+// the points of each cloud as they lie in memory; a null or empty cloud is an empty map
+void point_arrays(const std::vector<PointCloudConstPtr>& clouds, std::vector<const void*>& ptrs, std::vector<uint64_t>& sizes)
+{
+  ptrs.assign(clouds.size(), nullptr);
+  sizes.assign(clouds.size(), 0);
+  for (size_t i = 0; i < clouds.size(); ++i)
+    if (clouds[i] && !clouds[i]->points.empty()) {
+      ptrs[i] = clouds[i]->points.data();
+      sizes[i] = clouds[i]->points.size();
+    }
 }
 
 std::vector<float> pack_normals(const SurfaceNormals& nm)
@@ -447,18 +470,13 @@ std::vector<Eigen::Matrix4f> estimateMapsTransforms(const std::vector<PointCloud
 {
   if (clouds.empty()) return {};
   if (clouds.size() == 1) return {Eigen::Matrix4f::Identity()};
-  std::vector<std::vector<float>> packed(clouds.size());
-  std::vector<const float*> ptrs(clouds.size());
-  std::vector<uint64_t> sizes(clouds.size());
-  for (size_t i = 0; i < clouds.size(); ++i) {
-    packed[i] = pack(clouds[i].get());
-    ptrs[i] = packed[i].empty() ? nullptr : packed[i].data();
-    sizes[i] = packed[i].size() / 4;
-  }
+  std::vector<const void*> ptrs;
+  std::vector<uint64_t> sizes;
+  point_arrays(clouds, ptrs, sizes);
   const mm3d_params cp = to_c(params);
   std::vector<float> out(clouds.size() * 16);
   int n_out = 0;
-  check(mm3d_estimate_maps_transforms(context(), (int)clouds.size(), ptrs.data(), sizes.data(), &cp, out.data(), &n_out));
+  check(mm3d_estimate_maps_transforms_layout(context(), (int)clouds.size(), ptrs.data(), sizes.data(), &point_layout(), &cp, out.data(), &n_out));
   std::vector<Eigen::Matrix4f> r;
   for (int i = 0; i < n_out; ++i) r.push_back(to_matrix(out.data() + 16 * i));
   return r;
@@ -468,25 +486,28 @@ PointCloudPtr composeMaps(const std::vector<PointCloudConstPtr>& clouds, const s
 {
   if (clouds.empty()) return nullptr;
   if (clouds.size() != transforms.size()) throw std::runtime_error("composeMaps: clouds and transforms size must be the same.");
-  std::vector<std::vector<float>> packed(clouds.size());
-  std::vector<const float*> ptrs(clouds.size());
-  std::vector<uint64_t> sizes(clouds.size());
+  std::vector<const void*> ptrs;
+  std::vector<uint64_t> sizes;
+  point_arrays(clouds, ptrs, sizes);
   bool any = false;
-  for (size_t i = 0; i < clouds.size(); ++i) {
-    packed[i] = pack(clouds[i].get());
-    ptrs[i] = packed[i].empty() ? nullptr : packed[i].data();
-    sizes[i] = packed[i].size() / 4;
-    any = any || sizes[i] > 0;
-  }
+  for (uint64_t n : sizes) any = any || n > 0;
   if (!any) return PointCloudPtr(new PointCloud);
   std::vector<float> T(transforms.size() * 16);
   for (size_t i = 0; i < transforms.size(); ++i) std::memcpy(&T[16 * i], transforms[i].data(), 64);
-  float* out = nullptr;
+  void* out = nullptr;
   uint64_t n = 0;
-  const int rc = mm3d_compose_maps(context(), (int)clouds.size(), ptrs.data(), sizes.data(), (int)transforms.size(), T.data(), resolution, &out, &n);
+  const mm3d_layout& l = point_layout();
+  const int rc = mm3d_compose_maps_layout(context(), (int)clouds.size(), ptrs.data(), sizes.data(), &l, (int)transforms.size(), T.data(), resolution,
+                                          &l, &out, &n);
   if (rc == 1) return nullptr;
   check(rc);
-  PointCloudPtr r = unpack(out, n);
+  // the records are default-constructed points with x, y, z and rgba filled in, which is what unpack() builds
+  PointCloudPtr r(new PointCloud);
+  r->points.resize(n);
+  if (n) std::memcpy((void*)r->points.data(), out, n * sizeof(PointT));
+  r->width = (uint32_t)n;
+  r->height = 1;
+  r->is_dense = true;
   mm3d_free(out);
   return r;
 }
