@@ -121,6 +121,46 @@ int mm3d_compose_maps_layout(mm3d_ctx* ctx, int n_maps, const void* const* cloud
 int mm3d_maps_upload_layout(mm3d_ctx* ctx, int n_maps, const void* const* clouds, const uint64_t* n_points, const mm3d_layout* layout,
                             mm3d_maps** maps);
 
+/* ---- map set: resident maps that re-estimate only what changed (csrc/mapset.cu) ---------------------------------------
+ * An ordered list of slots, one per robot.  Each slot keeps its raw cloud on the device, the features computed from it and,
+ * for every pair, the last registration result.  It serves the reference's ROS node pattern (map_merge_node): each map
+ * callback replaces one slot, and the estimation and compositing timers run over all slots.
+ *
+ * Contract: after any sequence of updates and parameter changes, mm3d_mapset_estimate returns bit for bit what
+ * mm3d_estimate_maps_transforms returns on the slots' current clouds in slot order (n_out, empty slots and SAC_IA
+ * included), and mm3d_mapset_compose returns bit for bit what mm3d_compose_maps_layout returns.  Caching skips work; it
+ * never changes a result.
+ *   - A map's features are recomputed when its cloud changed (bitwise, after conversion to the packed layout).
+ *   - A pair is registered again when either of its maps changed.  Under MM3D_EST_SAC_IA it is also registered again
+ *     when the offset at which its draws start in the C rand() stream moved, because an earlier source map's keypoints
+ *     changed.
+ *   - Any field of mm3d_params that differs from the previous estimate recomputes everything.
+ *   - Cached state is committed only when a call succeeds; after an error the next estimate redoes what was pending.
+ * A malformed layout, a negative or repeated slot index, a NULL pointer where one is required, or a ctx other than the
+ * one the set was created on returns MM3D_ERR_ARG, launches nothing and leaves the set unchanged.
+ * A set is used by one thread at a time, like a context, and is freed before its context.  On an mm3d_create_multi context
+ * it runs on the first device. */
+typedef struct mm3d_mapset mm3d_mapset;
+/* a set with no slots */
+int mm3d_mapset_create(mm3d_ctx* ctx, mm3d_mapset** set);
+/* Replace the clouds of n slots (records in `layout`; a NULL cloud or 0 points is an empty cloud).  A slot index at or past
+ * the current count grows the set; slots in between are empty.  changed (optional, n ints): 1 when the slot's cloud differs
+ * from the resident one, bit for bit after conversion to the packed layout, or the call created the slot.  An unchanged
+ * slot keeps its resident cloud and everything computed from it. */
+int mm3d_mapset_update(mm3d_ctx* ctx, mm3d_mapset* set, int n, const int32_t* slots, const void* const* clouds, const uint64_t* n_points,
+                       const mm3d_layout* layout, int32_t* changed);
+/* number of slots (0 for NULL) */
+int mm3d_mapset_size(const mm3d_mapset* set);
+/* mm3d_estimate_maps_transforms over the slots; out_transforms has room for mm3d_mapset_size matrices.
+ * work (optional, 3 ints): maps whose features were computed, pairs registered, pairs reused.  With nothing changed since
+ * the previous estimate and the same params, no kernel is launched. */
+int mm3d_mapset_estimate(mm3d_ctx* ctx, mm3d_mapset* set, const mm3d_params* params, float* out_transforms, int* n_out, int32_t* work);
+/* mm3d_compose_maps_layout over the slots' resident clouds: 1 with *out = NULL when the set has no slots, MM3D_ERR_ARG when
+ * n_transforms differs from the slot count; *out = n_out records in out_layout (mm3d_free). */
+int mm3d_mapset_compose(mm3d_ctx* ctx, const mm3d_mapset* set, int n_transforms, const float* transforms, double resolution,
+                        const mm3d_layout* out_layout, void** out, uint64_t* n_out);
+void mm3d_mapset_free(mm3d_mapset* set);
+
 /* ---- low-level interface (features.h / matching.h) ------------------------ */
 /* index_leaf: voxel size the cloud was built with (MapMergingParams::resolution); 0 picks
  * radius / 8 (descriptor-style radii) or radius / 6 (normal-style radii), the reference's

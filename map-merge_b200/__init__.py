@@ -45,6 +45,7 @@ SYMBOLS = [
     "mm3d_knn", "mm3d_knn_tc_audit", "mm3d_create_multi", "mm3d_device_count", "mm3d_comm_id", "mm3d_comm_create", "mm3d_comm_destroy", "mm3d_comm_rank", "mm3d_comm_size",
     "mm3d_dist_block", "mm3d_dist_plan", "mm3d_estimate_maps_transforms_dist", "mm3d_estimate_resident_dist", "mm3d_compose_maps_dist",
     "mm3d_compose_resident_dist", "mm3d_estimate_maps_transforms_layout", "mm3d_compose_maps_layout", "mm3d_maps_upload_layout",
+    "mm3d_mapset_create", "mm3d_mapset_update", "mm3d_mapset_size", "mm3d_mapset_estimate", "mm3d_mapset_compose", "mm3d_mapset_free",
 ]
 COMM_ID_BYTES = 128
 
@@ -115,6 +116,8 @@ def lib():
         L.mm3d_compose_shard_size.argtypes = [C.c_void_p, u64p]
         L.mm3d_comm_destroy.argtypes = [C.c_void_p]
         L.mm3d_device_count.argtypes = [C.c_void_p]
+        L.mm3d_mapset_size.argtypes = [C.c_void_p]
+        L.mm3d_mapset_free.argtypes = [C.c_void_p]
         _lib = L
     return _lib
 
@@ -510,6 +513,12 @@ class Context:
         T = out[:no.value].reshape(-1, 4, 4).transpose(0, 2, 1).copy()
         return (T, dict(zip(STAGES, st.tolist()))) if stage_times else T
 
+    def mapset(self) -> "MapSet":
+        """An empty map set on this context (mm3d_mapset_create): resident maps that re-estimate only what changed."""
+        h = C.c_void_p()
+        self._check(self.L.mm3d_mapset_create(self.h, C.byref(h)))
+        return MapSet(self, h)
+
     def features_compute(self, maps: "Maps", first: int, count: int, params: Params):
         h = C.c_void_p()
         self._check(self.L.mm3d_features_compute(self.h, maps.h, int(first), int(count), C.byref(params), C.byref(h)))
@@ -637,6 +646,70 @@ class Features:
     def free(self):
         if self.h:
             self.ctx.L.mm3d_features_free(self.h)
+            self.h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
+class MapSet:
+    """mm3d_mapset: one slot per robot; each keeps its cloud, features and pair results on the device between calls.
+    estimate() and compose() return bit for bit what estimate_maps_transforms and compose_maps_layout return on the slots'
+    current clouds in slot order."""
+
+    def __init__(self, ctx: Context, h):
+        self.ctx, self.h = ctx, h
+
+    def __len__(self):
+        return int(self.ctx.L.mm3d_mapset_size(self.h))
+
+    def update(self, clouds: dict, layout: Layout | None = None) -> list:
+        """clouds = {slot: cloud or None}: float32[n, 4] points, or uint8[n, layout.point_step] records when a layout is
+        given.  Returns, per entry in the dict's order, whether the slot's cloud changed (bit for bit)."""
+        slots = [int(k) for k in clouds]
+        values = list(clouds.values())
+        if layout is None:
+            arrs, ptrs, ns = self.ctx._cloud_args(values)
+            layout = PACKED
+        else:
+            arrs, ptrs, ns = self.ctx._record_args(values, layout)
+        n = len(slots)
+        sl = (C.c_int32 * max(n, 1))(*slots)
+        changed = (C.c_int32 * max(n, 1))()
+        self.ctx._check(self.ctx.L.mm3d_mapset_update(self.ctx.h, self.h, n, sl, ptrs, ns, C.byref(layout), changed))
+        return [bool(changed[i]) for i in range(n)]
+
+    def estimate(self, params: Params, work: bool = False):
+        """Transforms as estimate_maps_transforms returns them; work=True also returns [maps whose features were computed,
+        pairs registered, pairs reused]."""
+        m = len(self)
+        out = np.zeros((max(m, 1), 16), np.float32); no = C.c_int(); w = (C.c_int32 * 3)()
+        self.ctx._check(self.ctx.L.mm3d_mapset_estimate(self.ctx.h, self.h, C.byref(params), out.ctypes.data_as(f32p), C.byref(no), w))
+        T = out[:no.value].reshape(-1, 4, 4).transpose(0, 2, 1).copy()
+        return (T, [int(x) for x in w]) if work else T
+
+    def compose(self, transforms, resolution, out_layout: Layout | None = None):
+        """compose_maps over the slots: float32[n, 4] points, or uint8[n, out_layout.point_step] records when out_layout is
+        given; None for a set without slots."""
+        T = np.asarray(transforms, np.float32).reshape(-1, 4, 4)
+        Tc = np.ascontiguousarray(T.transpose(0, 2, 1)) if len(T) else np.zeros((1, 16), np.float32)
+        layout = PACKED if out_layout is None else out_layout
+        out = C.c_void_p(); n = C.c_uint64()
+        rc = self.ctx.L.mm3d_mapset_compose(self.ctx.h, self.h, len(T), Tc.ctypes.data_as(f32p), C.c_double(resolution), C.byref(layout),
+                                            C.byref(out), C.byref(n))
+        if rc == 1:
+            return None
+        self.ctx._check(rc)
+        if out_layout is None:
+            return self.ctx._take(out, n.value * 4, np.float32, (-1, 4))
+        return self.ctx._take(out, n.value * layout.point_step, np.uint8, (-1, layout.point_step))
+
+    def free(self):
+        if self.h:
+            self.ctx.L.mm3d_mapset_free(self.h)
             self.h = C.c_void_p()
 
     def __del__(self):

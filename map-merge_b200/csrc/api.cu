@@ -81,16 +81,16 @@ double auto_leaf(double index_leaf, double radius, double ratio)
   return radius / ratio;
 }
 
+}  // namespace
+
+namespace mm3d {
+
 void check_supported(const mm3d_params& p)
 {
   if (p.keypoint_type != MM3D_KP_SIFT && p.keypoint_type != MM3D_KP_HARRIS) throw UnsupportedError("unsupported: unknown keypoint_type");
   if (p.descriptor_type < MM3D_DESC_PFH || p.descriptor_type > MM3D_DESC_SC3D) throw UnsupportedError("unsupported: unknown descriptor_type");
   if (p.estimation_method != MM3D_EST_MATCHING && p.estimation_method != MM3D_EST_SAC_IA) throw UnsupportedError("unsupported: unknown estimation_method");
 }
-
-}  // namespace
-
-namespace mm3d {
 
 namespace {
 struct PinnedPool {
@@ -415,26 +415,6 @@ int bad_layout(mm3d_ctx* ctx)
 }
 
 }  // namespace
-
-#define MM_TRY(ctx) \
-  if (!(ctx)) return MM3D_ERR_ARG; \
-  Ctx& c = (ctx)->c; \
-  try { \
-    MM_CUDA(cudaSetDevice(c.device));
-#define MM_CATCH \
-  } catch (const UnsupportedError& e) { \
-    c.err = e.what(); \
-    return MM3D_ERR_UNSUPPORTED; \
-  } catch (const CudaError& e) { \
-    c.err = e.what(); \
-    cudaGetLastError(); \
-    return MM3D_ERR_CUDA; \
-  } catch (const std::exception& e) { \
-    c.err = e.what(); \
-    cudaGetLastError(); \
-    return MM3D_ERR; \
-  } \
-  return MM3D_OK;
 
 extern "C" {
 

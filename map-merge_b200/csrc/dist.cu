@@ -364,6 +364,10 @@ std::vector<int> choose_splitters(const std::vector<unsigned long long>& hist, i
   return sp;
 }
 
+}  // namespace
+
+namespace mm3d {
+
 // One rank's part of composeMaps: local clouds already on the device.  Returns this rank's slice of the composed map on the
 // host (host_out_alloc, records in out_layout); the slices concatenated in rank order are the reference's output bit for bit.
 void dist_compose(Ctx& c, mm3d_comm* cm, const std::vector<CloudView>& local, const std::vector<const float*>& transforms_rowmajor,
@@ -476,6 +480,10 @@ bool skip_map(const float* colmajor, const void* cloud, uint64_t n, float* rowma
     if (!(std::fabs(rowmajor[k]) <= 1e-5f)) zero = false;
   return zero || !cloud || n == 0;
 }
+
+}  // namespace mm3d
+
+namespace {
 
 // run fn(rank) on one host thread per device of the team; the first error wins
 template <typename F>

@@ -827,14 +827,15 @@ struct GlibcRand {
 
 void sac_ia_batch(Ctx& c, const std::vector<CloudView>& keypoints, const std::vector<const float*>& desc, int dim,
                   const std::vector<PairJob>& all_pairs, const std::vector<int>& wanted, double min_sample_distance, double max_corr_dist,
-                  int max_iterations, unsigned long long rand_skip, std::vector<SacOut>& out)
+                  int max_iterations, unsigned long long rand_skip, std::vector<SacOut>& out, std::vector<unsigned long long>* starts)
 {
   out.assign(wanted.size(), SacOut());
   for (SacOut& o : out) {
     for (int k = 0; k < 16; ++k) o.T[k] = (k % 5 == 0) ? 1.f : 0.f;  // align() leaves the identity guess when nothing is scored
     o.rand_calls = 0;
   }
-  if (wanted.empty() || max_iterations <= 0) return;
+  if (starts) starts->assign(all_pairs.size(), rand_skip);
+  if ((wanted.empty() && !starts) || max_iterations <= 0) return;
   const int M = (int)keypoints.size();
   const int n_it = max_iterations;
   // host copies of the keypoints: the sample selection is sequential and touches only a few points per draw
@@ -858,6 +859,7 @@ void sac_ia_batch(Ctx& c, const std::vector<CloudView>& keypoints, const std::ve
     const PairJob& pj = all_pairs[pi];
     const int ns = keypoints[pj.a].n, nt = keypoints[pj.b].n;
     const int slot = slot_of_pair[pi];
+    if (starts) (*starts)[pi] = rng.calls;
     if (ns < 3 || nt == 0) {
       if (slot >= 0) out[slot].rand_calls = rng.calls;
       continue;

@@ -827,10 +827,13 @@ struct SacOut {
   unsigned long long rand_calls;  // rand() calls consumed up to and including this pair
   std::vector<float> errors;      // per-iteration error metric
 };
-// all_pairs: the complete row-major pair list (the rand() stream runs through all of it); wanted: indices into all_pairs
+// all_pairs: the complete row-major pair list (the rand() stream runs through all of it); wanted: indices into all_pairs.
+// starts (optional): per entry of all_pairs, the rand() calls made before that pair's draws.  With wanted empty the call
+// only walks the stream on the host and launches nothing.
 void sac_ia_batch(Ctx& c, const std::vector<CloudView>& keypoints, const std::vector<const float*>& desc, int dim,
                   const std::vector<PairJob>& all_pairs, const std::vector<int>& wanted, double min_sample_distance, double max_corr_dist,
-                  int max_iterations, unsigned long long rand_skip, std::vector<SacOut>& out);
+                  int max_iterations, unsigned long long rand_skip, std::vector<SacOut>& out,
+                  std::vector<unsigned long long>* starts = nullptr);
 
 // icp.cu — K11, K12
 // Reach grid of a target cloud: per voxel of the (margin-extended) index grid a LOWER bound, in voxel units squared, of the

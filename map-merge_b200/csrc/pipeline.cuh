@@ -51,6 +51,8 @@ void compute_features(Ctx& c, const std::vector<CloudView>& raw, const mm3d_para
 void register_pairs(Ctx& c, const std::vector<FeatView>& f, int dim, const std::vector<PairJob>& jobs, const mm3d_params& p,
                     std::vector<PairOut>& out, float* stage_ms);
 int desc_dim(const mm3d_params& p);
+// throws UnsupportedError for an enum value the library does not know
+void check_supported(const mm3d_params& p);
 std::vector<FeatView> feat_views(const std::vector<MapFeat>& f);
 void to_colmajor(const float* rm, float* cm);
 void from_colmajor(const float* cm, float* rm);
@@ -67,6 +69,12 @@ DCloud upload_cloud(Ctx& c, const float* pts, uint64_t n);  // one cloud in the 
 void* download_records(Ctx& c, const float4* pts, size_t n, const mm3d_layout& l);
 void staging_release(Ctx& c);
 
+// dist.cu: one rank's part of composeMaps on device clouds (cm = NULL: a single rank); *out = records in out_layout
+// (host_out_alloc)
+void dist_compose(Ctx& c, mm3d_comm* cm, const std::vector<CloudView>& local, const std::vector<const float*>& transforms_rowmajor,
+                  double resolution, const mm3d_layout& out_layout, void** out, uint64_t* n_out);
+// composeMaps' skip rule (map_merging.cpp:293-295): true for a zero transform or an empty cloud; rowmajor = the transform
+bool skip_map(const float* colmajor, const void* cloud, uint64_t n, float* rowmajor);
 // dist.cu: the high-level calls over the devices of a mm3d_create_multi context (one host thread per device)
 int team_size(const mm3d_ctx* ctx);
 int team_estimate(mm3d_ctx* master, int n_maps, const void* const* clouds, const uint64_t* n_points, const mm3d_layout& layout,
@@ -75,6 +83,27 @@ void team_compose(mm3d_ctx* master, int n_maps, const void* const* clouds, const
                   const float* transforms, double resolution, const mm3d_layout& out_layout, void** out, uint64_t* n_out);
 
 }  // namespace mm3d
+
+// Body of a C ABI entry point: errors thrown by the pipeline become status codes and the context's last error.
+#define MM_TRY(ctx) \
+  if (!(ctx)) return MM3D_ERR_ARG; \
+  Ctx& c = (ctx)->c; \
+  try { \
+    MM_CUDA(cudaSetDevice(c.device));
+#define MM_CATCH \
+  } catch (const UnsupportedError& e) { \
+    c.err = e.what(); \
+    return MM3D_ERR_UNSUPPORTED; \
+  } catch (const CudaError& e) { \
+    c.err = e.what(); \
+    cudaGetLastError(); \
+    return MM3D_ERR_CUDA; \
+  } catch (const std::exception& e) { \
+    c.err = e.what(); \
+    cudaGetLastError(); \
+    return MM3D_ERR; \
+  } \
+  return MM3D_OK;
 
 struct mm3d_features {
   std::vector<mm3d::MapFeat> maps;
