@@ -166,17 +166,31 @@ __device__ __forceinline__ float block27_any(const GridView& g, int vx, int vy, 
   return best;
 }
 
+// Gap slack of the voxel geometry, in voxels, for a query at voxel coordinates (fx, fy, fz) = fl(q * inv_leaf).  The query's
+// coordinate and a point's row, floor(fl(p * inv_leaf)), are each rounded by up to half an ulp of the voxel coordinate, so
+// the true gap between the query and a neighbouring row or cell can be smaller than the computed one by up to about
+// |f| * 2^-23 per axis: 5e-4 voxel at 500 m from the origin with a 0.1 m leaf.  Twice that bound, summed over the axes:
+__device__ __forceinline__ float voxel_slack(float fx, float fy, float fz)
+{
+  return (fabsf(fx) + fabsf(fy) + fabsf(fz) + 1.0f) * 2.384185791015625e-7f;  // 2^-22
+}
+
 // The 3 x 3 x 3 voxel block around the query in an index with one-voxel cells: nine (z, y) rows of three cells each, every
 // row one contiguous run of points.  All nine run bounds are loaded up front (independent loads), rows are skipped when
 // their slab distance already exceeds the running best.  Every point outside the block is at least one voxel away, so a
 // best closer than that is the exact nearest neighbour (*certain); otherwise the caller falls back to the general search.
+// Both tests take the slab distances and the one voxel less voxel_slack, so they hold at any distance from the origin.
 __device__ __forceinline__ bool nearest_block27(const GridView& g, float qx, float qy, float qz, double bound, int guess_slot, int* out_idx,
                                                 float* out_d2, float4* out_pt, int* out_slot, bool* certain)
 {
   const float fx = qx * g.inv_leaf, fy = qy * g.inv_leaf, fz = qz * g.inv_leaf;
+  const float slack = voxel_slack(fx, fy, fz);
   const float flx = floorf(fx), fly = floorf(fy), flz = floorf(fz);
   const int vx = (int)flx - g.min_b[0], vy = (int)fly - g.min_b[1], vz = (int)flz - g.min_b[2];
   const float ay = fy - fly, az = fz - flz;  // position inside the voxel, voxel units
+  // least gaps to the rows below and above, voxels
+  const float ylo = fmaxf(ay - slack, 0.0f), yhi = fmaxf(1.0f - ay - slack, 0.0f);
+  const float zlo = fmaxf(az - slack, 0.0f), zhi = fmaxf(1.0f - az - slack, 0.0f);
   bool found = false;
   float best = 0.0f;
   int best_idx = 0x7fffffff, best_slot = -1;
@@ -212,8 +226,8 @@ __device__ __forceinline__ bool nearest_block27(const GridView& g, float qx, flo
 #pragma unroll
   for (int t = 0; t < 9; ++t) {
     const int dz = t / 3 - 1, dy = t % 3 - 1;
-    const float zd = dz < 0 ? az : (dz > 0 ? 1.0f - az : 0.0f);
-    const float yd = dy < 0 ? ay : (dy > 0 ? 1.0f - ay : 0.0f);
+    const float zd = dz < 0 ? zlo : (dz > 0 ? zhi : 0.0f);
+    const float yd = dy < 0 ? ylo : (dy > 0 ? yhi : 0.0f);
     if (zd * zd + yd * yd > bestv) continue;
     for (int k = rs[t]; k < re[t]; ++k) {
       const float4 p = g.pts[k];
@@ -230,7 +244,8 @@ __device__ __forceinline__ bool nearest_block27(const GridView& g, float qx, flo
       }
     }
   }
-  *certain = found && best * inv2 < 0.999f;
+  const float outside = fmaxf(1.0f - slack, 0.0f);  // least gap to a point outside the block, voxels
+  *certain = found && best * inv2 < 0.999f * outside * outside;
   *out_idx = best_idx;
   *out_d2 = best;
   *out_pt = best_pt;
@@ -273,15 +288,19 @@ __device__ __forceinline__ bool tile_nearest(TileNn& sh, const GridView& g, cons
   if (live) {
     float r2 = (float)bound;  // radius^2 phase 2 would have to search
     bool rejected = false, block_has_points = true;
+    // the reach grid's bounds and phase 2's row bounds count whole cells; the true gaps may be short of them by the
+    // rounding slack on each axis, at most 2 * slack along any direction
+    const float slack2 = 2.0f * voxel_slack(qx * g.inv_leaf, qy * g.inv_leaf, qz * g.inv_leaf);
     if (r.lb2) {
       int lb2 = 0;
       const float bound_v = (float)bound * g.inv_leaf * g.inv_leaf;  // bound in voxel units, squared
       const bool inside = reach_lookup(g, r, qx, qy, qz, &lb2);
       // outside the grid: farther than the margin from every occupied voxel, i.e. lower bound >= none
+      // (sqrt(lb) - slack2)^2 >= lb - slack2 * (lb + 1), as 2 sqrt(lb) <= lb + 1
       const float lb = inside ? (float)lb2 : (float)r.none;
-      if (lb > bound_v * 1.001f + 0.01f) rejected = true;
+      if (lb - slack2 * (lb + 1.0f) > bound_v * 1.001f + 0.01f) rejected = true;
       if (inside && lb2 < r.none) {
-        const float ub = sqrtf((float)lb2) + 3.4642f;  // + twice the voxel diagonal
+        const float ub = sqrtf((float)lb2) + 3.4642f + slack2;  // + twice the voxel diagonal
         r2 = fminf(r2, (ub * ub * 1.001f + 0.01f) * g.leaf * g.leaf);
       }
       block_has_points = inside && lb2 == 0;  // lower bound 0 <=> an occupied voxel inside the 3 x 3 x 3 block
@@ -308,7 +327,9 @@ __device__ __forceinline__ bool tile_nearest(TileNn& sh, const GridView& g, cons
       if (!certain) {
         pending = true;
         hit = false;
-        const float r2w = r2 * 1.00001f + 1e-12f;  // strict < inside the walk: widen by a hair
+        // strict < inside the walk: widen by a hair; and by the slack, which the walk's whole-cell row bounds do not have
+        const float rw = sqrtf(r2 * 1.00001f + 1e-12f) + slack2 * g.leaf;
+        const float r2w = rw * rw;
         sh.q[tid] = make_float4(qx, qy, qz, r2w);
         if (r2w * g.inv_leaf * g.inv_leaf <= 12.25f) sh.todo[atomicAdd(&sh.n_todo, 1)] = tid;  // radius <= 3.5 voxels: at most 11 x 11 rows
         else sh.todo_large[atomicAdd(&sh.n_todo_large, 1)] = tid;

@@ -100,13 +100,21 @@ __global__ void geom_kernel(const CloudView* __restrict__ clouds, const uint32_t
       const long long dx = (long long)ex + 1, dy = (long long)ey + 1, dz = (long long)ez + 1;
       if (!(ex < 3e9f) || !(ey < 3e9f) || !(ez < 3e9f) || dx * dy * dz > 2147483647LL) pass = true;
     }
-    if (pass) {
-      g.passthrough = 1;
-    } else {
+    g.passthrough = pass ? 1 : 0;
+    // The box in voxels.  Past the guard the output is the input, but neighbour indexes over it still need the box; it is
+    // left at zero when its voxel coordinates do not fit in int32.
+    bool fits = leaf > 0.0f;
+    for (int k = 0; k < 3; ++k) {
+      const float lo = floorf(mn[k] * inv), hi = floorf(mx[k] * inv);
+      fits = fits && lo >= -2147483648.0f && hi < 2147483647.0f && (long long)hi - (long long)lo < 2147483647LL;
+    }
+    if (!pass || fits) {
       for (int k = 0; k < 3; ++k) {
         g.min_b[k] = (int)floorf(mn[k] * inv);
         g.div_b[k] = (int)floorf(mx[k] * inv) - g.min_b[k] + 1;
       }
+    }
+    if (!pass) {
       const long long cells = (long long)g.div_b[0] * g.div_b[1] * g.div_b[2];
       int nb = 1;
       while (nb < 32 && (1LL << nb) < cells) ++nb;
@@ -465,7 +473,11 @@ void build_index_batch(Ctx& c, const std::vector<CloudView>& clouds, float leaf,
   else compute_geom(c, clouds, dviews, leaf, geom, dgeom);
   std::vector<IndexGeom> ig(M);
   for (int m = 0; m < M; ++m) {
-    if (geom[m].passthrough && clouds[m].n > 0) throw std::runtime_error("build_index: leaf too small for the cloud extent");
+    // Past pcl::VoxelGrid's overflow guard the index still works from the box (coarsened below like any large one), unless
+    // the box's voxel coordinates do not fit in int32 or the cloud kept non-finite points, which have no cell.
+    if (geom[m].passthrough && clouds[m].n > 0 && (geom[m].div_b[0] <= 0 || geom[m].nonfinite > 0))
+      throw std::runtime_error(geom[m].nonfinite > 0 ? "build_index: non-finite points in a cloud past the voxel-grid overflow guard"
+                                                     : "build_index: voxel coordinates of the cloud do not fit in int32");
     int sh[3] = {sx, sy, sz};
     IndexGeom& g = ig[m];
     for (;;) {
