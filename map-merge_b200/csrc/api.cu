@@ -1,6 +1,7 @@
 // api.cu — the C ABI (include/mm3d.h) and the orchestration of the hot path:
 // stage-major per-map loops and the all-pairs loop of
 // map_merge_3d/src/map_merging.cpp:188-275, each stage one batched launch set.
+#include <algorithm>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -269,16 +270,15 @@ void register_pairs(Ctx& c, const std::vector<FeatView>& f, int dim, const std::
     // estimateTransformFromDescriptorsSets(min_sample_distance = inlier_threshold, max_correspondence_distance, max_iterations)
     // (matching.cpp:242-247).  The C rand() stream runs through the complete row-major pair list of the feature set.
     tm.begin(6);
-    std::vector<PairJob> all_pairs;
-    for (int i = 0; i < M - 1; ++i)
-      for (int j2 = i + 1; j2 < M; ++j2)
-        if (nk[i] > 0 && nk[j2] > 0) all_pairs.push_back(PairJob{i, j2});
-    std::vector<int> wanted(P, -1);
-    for (int k = 0; k < P; ++k)
-      for (size_t a = 0; a < all_pairs.size(); ++a)
-        if (all_pairs[a].a == jobs[k].a && all_pairs[a].b == jobs[k].b) wanted[k] = (int)a;
-    for (int k = 0; k < P; ++k)
-      if (wanted[k] < 0) throw std::runtime_error("register_pairs(SAC_IA): pair is not in the row-major pair list (i < j, both with keypoints)");
+    const std::vector<PairJob> all_pairs = row_major_pairs(nk);
+    auto before = [](const PairJob& x, const PairJob& y) { return x.a < y.a || (x.a == y.a && x.b < y.b); };  // the list's order
+    std::vector<int> wanted(P);
+    for (int k = 0; k < P; ++k) {
+      const auto it = std::lower_bound(all_pairs.begin(), all_pairs.end(), jobs[k], before);
+      if (it == all_pairs.end() || it->a != jobs[k].a || it->b != jobs[k].b)
+        throw std::runtime_error("register_pairs(SAC_IA): pair is not in the row-major pair list (i < j, both with keypoints)");
+      wanted[k] = (int)(it - all_pairs.begin());
+    }
     std::vector<SacOut> so;
     sac_ia_batch(c, kps, desc, dim, all_pairs, wanted, p.inlier_threshold, p.max_correspondence_distance, p.max_iterations, 0, so);
     for (int k = 0; k < P; ++k) {
@@ -346,9 +346,9 @@ void register_pairs(Ctx& c, const std::vector<FeatView>& f, int dim, const std::
   c.sync();
 }
 
-int desc_dim(const mm3d_params& p)
+int desc_dim(int descriptor_type)
 {
-  switch (p.descriptor_type) {
+  switch (descriptor_type) {
     case MM3D_DESC_SHOT: return 1344;
     case MM3D_DESC_PFH: return 125;
     case MM3D_DESC_PFHRGB: return 250;
@@ -365,48 +365,16 @@ std::vector<FeatView> feat_views(const std::vector<MapFeat>& f)
   return v;
 }
 
+std::vector<CloudView> views(const std::vector<DCloud>& d)
+{
+  std::vector<CloudView> v(d.size());
+  for (size_t m = 0; m < d.size(); ++m) v[m] = d[m].view();
+  return v;
+}
+
 }  // namespace mm3d
 
 namespace {
-
-// returns number of transforms written
-int estimate_from_views(Ctx& c, const std::vector<CloudView>& raw, const mm3d_params& p, float* out_transforms, float* stage_ms)
-{
-  const int M = (int)raw.size();
-  if (M == 0) return 0;
-  if (M == 1) {
-    const float id[16] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1};
-    memcpy(out_transforms, id, sizeof(id));
-    return 1;
-  }
-  std::vector<MapFeat> f;
-  compute_features(c, raw, p, f, stage_ms);
-  std::vector<PairJob> jobs;
-  for (int i = 0; i < M - 1; ++i)
-    for (int j = i + 1; j < M; ++j)
-      if (f[i].keypoints.n > 0 && f[j].keypoints.n > 0) jobs.push_back(PairJob{i, j});
-  std::vector<PairOut> po;
-  register_pairs(c, feat_views(f), desc_dim(p), jobs, p, po, stage_ms);
-  std::vector<HostEstimate> est(jobs.size());
-  for (size_t k = 0; k < jobs.size(); ++k) {
-    est[k].source_idx = (size_t)jobs[k].a;
-    est[k].target_idx = (size_t)jobs[k].b;
-    memcpy(est[k].T, po[k].T, sizeof(float) * 16);
-    est[k].confidence = po[k].confidence;
-  }
-  std::vector<std::vector<float>> g = compute_global_transforms(est, p.confidence_threshold, nullptr, nullptr, nullptr, nullptr);
-  for (size_t i = 0; i < g.size(); ++i) to_colmajor(g[i].data(), out_transforms + 16 * i);
-  HostProf& hp = host_prof();
-  if (hp.on) {
-    fprintf(stderr, "[mm3d host] buffer allocations %ld calls %.2f ms (%.1f MB), cudaFreeAsync %ld calls %.2f ms, sync %ld calls %.2f ms, "
-            "small copies %ld calls %.2f ms; block cache holds %.1f MB\n", hp.n_alloc, hp.alloc_ms, hp.alloc_bytes / 1e6, hp.n_free, hp.free_ms,
-            hp.n_sync, hp.sync_ms, hp.n_copy, hp.copy_ms, c.cache->held_bytes / 1e6);
-    const bool on = hp.on;
-    hp = HostProf();
-    hp.on = on;
-  }
-  return (int)g.size();
-}
 
 int bad_layout(mm3d_ctx* ctx)
 {
@@ -503,9 +471,7 @@ int mm3d_estimate_maps_transforms_layout(mm3d_ctx* ctx, int n_maps, const void* 
   // the degenerate cases never touch the device (map_merging.cpp:192-197)
   if (n_maps == 0) return MM3D_OK;
   if (n_maps == 1) {
-    const float id[16] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1};
-    memcpy(out_transforms, id, sizeof(id));
-    *n_out = 1;
+    *n_out = one_map_identity(out_transforms);
     return MM3D_OK;
   }
   MM_TRY(ctx)
@@ -514,9 +480,7 @@ int mm3d_estimate_maps_transforms_layout(mm3d_ctx* ctx, int n_maps, const void* 
     return MM3D_OK;
   }
   std::vector<DCloud> d = upload_clouds(c, std::vector<const void*>(clouds, clouds + n_maps), std::vector<uint64_t>(n_points, n_points + n_maps), *layout);
-  std::vector<CloudView> v(n_maps);
-  for (int m = 0; m < n_maps; ++m) v[m] = d[m].view();
-  *n_out = estimate_from_views(c, v, *params, out_transforms, nullptr);
+  *n_out = dist_estimate(c, nullptr, n_maps, views(d), *params, out_transforms, nullptr, nullptr);
   c.sync();
   MM_CATCH
 }
@@ -554,34 +518,9 @@ int mm3d_compose_maps_layout(mm3d_ctx* ctx, int n_maps, const void* const* cloud
     team_compose(ctx, n_maps, clouds, n_points, *in_layout, transforms, resolution, *out_layout, out, n_out);
     return MM3D_OK;
   }
-  std::vector<const void*> src;
-  std::vector<uint64_t> cnt;
-  std::vector<std::vector<float>> tr;
-  for (int m = 0; m < n_maps; ++m) {
-    float rm[16];
-    from_colmajor(transforms + 16 * m, rm);
-    bool zero = true;  // Eigen isZero(): every |a_ij| <= 1e-5
-    for (int k = 0; k < 16; ++k)
-      if (!(std::fabs(rm[k]) <= 1e-5f)) zero = false;
-    if (zero || !clouds[m] || n_points[m] == 0) continue;
-    src.push_back(clouds[m]);
-    cnt.push_back(n_points[m]);
-    tr.emplace_back(rm, rm + 16);
-  }
-  std::vector<DCloud> d = upload_clouds(c, src, cnt, *in_layout);
-  std::vector<CloudView> v;
-  std::vector<const float*> tp;
-  for (size_t i = 0; i < d.size(); ++i) {
-    v.push_back(d[i].view());
-    tp.push_back(tr[i].data());
-  }
-  DCloud cat;
-  transform_concat(c, v, tp, cat);
-  std::vector<DCloud> res;
-  voxel_downsample_batch(c, {cat.view()}, (float)resolution, res, nullptr);
-  *out = download_records(c, res[0].pts.p, (size_t)res[0].n, *out_layout);
-  *n_out = (uint64_t)res[0].n;
-  c.sync();
+  KeptMaps k;
+  std::vector<DCloud> d = upload_kept(c, clouds, n_points, 0, n_maps, transforms, *in_layout, k);
+  dist_compose(c, nullptr, views(d), k.transforms(), resolution, *out_layout, out, n_out);
   MM_CATCH
 }
 
@@ -683,7 +622,7 @@ int mm3d_descriptors(mm3d_ctx* ctx, const float* pts, uint64_t n, const float* n
   std::vector<DIndex> idx;
   build_index_batch(c, {d.view()}, (float)auto_leaf(index_leaf, radius, 8.0), 2, 0, 0, idx);
   std::vector<DBuf<float>> desc, sp;
-  const int D = type == MM3D_DESC_SHOT ? 1344 : (type == MM3D_DESC_PFH ? 125 : (type == MM3D_DESC_PFHRGB ? 250 : (type == MM3D_DESC_RSD ? 2 : (type == MM3D_DESC_SC3D ? 1980 : 33))));
+  const int D = desc_dim(type);
   if (type == MM3D_DESC_RSD || type == MM3D_DESC_SC3D) {
     if (type == MM3D_DESC_RSD) rsd_batch(c, {d.view()}, idx, {nm.p}, kp, radius, desc);
     else sc3d_batch(c, {d.view()}, idx, {nm.p}, kp, radius, desc);
@@ -972,26 +911,10 @@ int mm3d_compose_shard_begin(mm3d_ctx* ctx, int n_maps, const float* const* clou
     return MM3D_ERR_ARG;
   }
   MM_TRY(ctx)
-  std::vector<DCloud> d;
-  std::vector<std::vector<float>> tr;
-  for (int m = 0; m < n_maps; ++m) {
-    float rm[16];
-    from_colmajor(transforms + 16 * m, rm);
-    bool zero = true;
-    for (int k = 0; k < 16; ++k)
-      if (!(std::fabs(rm[k]) <= 1e-5f)) zero = false;
-    if (zero || !clouds[m] || n_points[m] == 0) continue;
-    d.push_back(upload_cloud(c, clouds[m], n_points[m]));
-    tr.emplace_back(rm, rm + 16);
-  }
-  std::vector<CloudView> v;
-  std::vector<const float*> tp;
-  for (size_t i = 0; i < d.size(); ++i) {
-    v.push_back(d[i].view());
-    tp.push_back(tr[i].data());
-  }
+  KeptMaps k;
+  std::vector<DCloud> d = upload_kept(c, (const void* const*)clouds, n_points, 0, n_maps, transforms, kPackedLayout, k);
   std::unique_ptr<mm3d_shard> s(new mm3d_shard);
-  transform_concat(c, v, tp, s->cloud);
+  transform_concat(c, views(d), k.transforms(), s->cloud);
   compose_bbox(c, s->cloud, bbox);
   *shard = s.release();
   MM_CATCH
@@ -1194,9 +1117,7 @@ int mm3d_estimate_resident(mm3d_ctx* ctx, const mm3d_maps* maps, const mm3d_para
   MM_TRY(ctx)
   if (stage_ms)
     for (int i = 0; i < 10; ++i) stage_ms[i] = 0.f;
-  std::vector<CloudView> v(maps->clouds.size());
-  for (size_t m = 0; m < v.size(); ++m) v[m] = maps->clouds[m].view();
-  *n_out = estimate_from_views(c, v, *params, out_transforms, stage_ms);
+  *n_out = dist_estimate(c, nullptr, (int)maps->clouds.size(), views(maps->clouds), *params, out_transforms, nullptr, stage_ms);
   c.sync();
   MM_CATCH
 }

@@ -23,7 +23,6 @@
 #include <nccl.h>
 
 #include <algorithm>
-#include <chrono>
 #include <cstring>
 #include <mutex>
 #include <numeric>
@@ -170,7 +169,15 @@ void lpt_assign(const std::vector<PairJob>& pairs, const std::vector<double>& co
   }
 }
 
-double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+// the rank that registers each pair of the row-major list
+std::vector<int> pair_owners(const std::vector<PairJob>& pairs, const std::vector<int>& npt, const std::vector<int>& nkp, int dim, int world)
+{
+  std::vector<double> cost(pairs.size());
+  for (size_t k = 0; k < pairs.size(); ++k) cost[k] = pair_cost(npt[pairs[k].a], npt[pairs[k].b], nkp[pairs[k].a], nkp[pairs[k].b], dim);
+  std::vector<int> owner;
+  lpt_assign(pairs, cost, world, owner);
+  return owner;
+}
 
 struct Phases {
   Ctx& c;
@@ -181,14 +188,14 @@ struct Phases {
     if (ms) {
       for (int i = 0; i < 5; ++i) ms[i] = 0.f;
       c.sync();
-      t0 = now_ms();
+      t0 = host_now_ms();
     }
   }
   void mark(int k)
   {
     if (!ms) return;
     c.sync();
-    const double t = now_ms();
+    const double t = host_now_ms();
     ms[k] += (float)(t - t0);
     t0 = t;
   }
@@ -196,59 +203,38 @@ struct Phases {
 
 constexpr int RES_W = 22;  // per pair: 16 transform floats, confidence (double bits), contribution count, 4 stats
 
-// One rank's part of estimateMapsTransforms.  local = this rank's block of raw clouds (device).  Returns the number of
-// transforms written (every rank gets all of them).
-int dist_estimate(Ctx& c, mm3d_comm* cm, int n_maps, const std::vector<CloudView>& local, const mm3d_params& p, float* out_transforms,
-                  float* phase_ms)
+// B + C of dist_estimate: every rank's sizes, then {cloud, keypoints, descriptors} of every map.  Per map one chunk
+// [points | keypoints | descriptors] in `all`, chunks padded to 256 bytes, rank r's chunks contiguous: rank r broadcasts
+// exactly its own region.  Returns views into `all`.
+std::vector<FeatView> exchange_features(Ctx& c, mm3d_comm* cm, int M, const std::vector<MapFeat>& f, int dim, DBuf<float>& all,
+                                        std::vector<int>& npt, std::vector<int>& nkp)
 {
-  const int W = cm ? cm->world : 1, R = cm ? cm->rank : 0;
-  const int M = n_maps;
-  if (M == 0) return 0;
-  if (M == 1) {
-    const float id[16] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1};
-    memcpy(out_transforms, id, sizeof(id));
-    return 1;
-  }
-  const int per = block_per(M, W);
+  const int W = cm->world, R = cm->rank, per = block_per(M, W);
   int first, count;
   block_of(R, W, M, &first, &count);
-  if ((int)local.size() != count) throw std::runtime_error("estimateMapsTransforms (multi-GPU): this rank's block holds " + std::to_string(count) + " maps");
-  Phases ph(c, phase_ms);
-
-  // ---- A: feature pipeline of the own block
-  std::vector<MapFeat> f;
-  compute_features(c, local, p, f, nullptr);
-  const int dim = desc_dim(p);
-  ph.mark(0);
-
-  // ---- B: sizes of every map
   std::vector<int> sz((size_t)W * per * 2, 0);
   for (int m = 0; m < count; ++m) {
     sz[((size_t)R * per + m) * 2] = f[m].cloud.n;
     sz[((size_t)R * per + m) * 2 + 1] = f[m].keypoints.n;
   }
-  if (W > 1) {
+  {
     DBuf<int> dsz(c, sz.size());
     dsz.upload(c, sz.data(), sz.size());
     MM_NCCL(nccl().AllGather(dsz.p + (size_t)R * per * 2, dsz.p, (size_t)per * 2, ncclInt32, cm->comm, c.stream));
     dsz.download(c, sz.data(), sz.size());
     c.sync();
   }
-  std::vector<int> npt(M), nkp(M);
   for (int m = 0; m < M; ++m) {
     const int r = std::min(m / per, W - 1), l = m - r * per;
     npt[m] = sz[((size_t)r * per + l) * 2];
     nkp[m] = sz[((size_t)r * per + l) * 2 + 1];
   }
-
-  // ---- C: exchange {cloud, keypoints, descriptors}; per map one chunk [points | keypoints | descriptors], chunks padded to
-  // 256 bytes, rank r's chunks contiguous: rank r broadcasts exactly its own region.
   std::vector<size_t> off(M + 1, 0);
   for (int m = 0; m < M; ++m) {
     const size_t floats = 4 * (size_t)npt[m] + 4 * (size_t)nkp[m] + (size_t)dim * nkp[m];
     off[m + 1] = off[m] + ((floats + 63) / 64) * 64;
   }
-  DBuf<float> all(c, off[M] + 64);
+  all.alloc(c, off[M] + 64);
   for (int m = 0; m < count; ++m) {
     float* base = all.p + off[first + m];
     if (f[m].cloud.n) MM_CUDA(cudaMemcpyAsync(base, f[m].cloud.pts.p, (size_t)f[m].cloud.n * 16, cudaMemcpyDeviceToDevice, c.stream));
@@ -258,17 +244,14 @@ int dist_estimate(Ctx& c, mm3d_comm* cm, int n_maps, const std::vector<CloudView
                               cudaMemcpyDeviceToDevice, c.stream));
     }
   }
-  if (W > 1) {
-    MM_NCCL(nccl().GroupStart());
-    for (int r = 0; r < W; ++r) {
-      int rf, rc;
-      block_of(r, W, M, &rf, &rc);
-      const size_t cnt = off[rf + rc] - off[rf];
-      if (cnt) MM_NCCL(nccl().Broadcast(all.p + off[rf], all.p + off[rf], cnt, ncclFloat, r, cm->comm, c.stream));
-    }
-    MM_NCCL(nccl().GroupEnd());
+  MM_NCCL(nccl().GroupStart());
+  for (int r = 0; r < W; ++r) {
+    int rf, rc;
+    block_of(r, W, M, &rf, &rc);
+    const size_t cnt = off[rf + rc] - off[rf];
+    if (cnt) MM_NCCL(nccl().Broadcast(all.p + off[rf], all.p + off[rf], cnt, ncclFloat, r, cm->comm, c.stream));
   }
-  f.clear();  // the views below point into `all`
+  MM_NCCL(nccl().GroupEnd());
   std::vector<FeatView> views(M);
   for (int m = 0; m < M; ++m) {
     const float* base = all.p + off[m];
@@ -276,18 +259,70 @@ int dist_estimate(Ctx& c, mm3d_comm* cm, int n_maps, const std::vector<CloudView
     views[m].keypoints = CloudView{(const float4*)(base + 4 * (size_t)npt[m]), nkp[m]};
     views[m].desc = base + 4 * (size_t)(npt[m] + nkp[m]);
   }
+  return views;
+}
+
+// Balanced key-range splitters from the all-reduced bucket histogram: splitters[r] <= bucket < splitters[r + 1] goes to rank r.
+std::vector<int> choose_splitters(const std::vector<unsigned long long>& hist, int world)
+{
+  const int nb = (int)hist.size();
+  std::vector<unsigned long long> cum(nb);
+  unsigned long long run = 0;
+  for (int i = 0; i < nb; ++i) { run += hist[i]; cum[i] = run; }
+  const unsigned long long total = run;
+  std::vector<int> sp(world + 1, 0);
+  sp[world] = nb;
+  for (int r = 1; r < world; ++r) {
+    const unsigned long long target = total * (unsigned long long)r / (unsigned long long)world;
+    int pos = (int)(std::lower_bound(cum.begin(), cum.end(), target) - cum.begin());
+    pos += total ? 1 : 0;
+    sp[r] = std::min(std::max(pos, sp[r - 1]), nb);
+  }
+  return sp;
+}
+
+}  // namespace
+
+namespace mm3d {
+
+int dist_estimate(Ctx& c, mm3d_comm* cm, int n_maps, const std::vector<CloudView>& local, const mm3d_params& p, float* out_transforms,
+                  float* phase_ms, float* stage_ms)
+{
+  const int W = cm ? cm->world : 1, R = cm ? cm->rank : 0;
+  const int M = n_maps;
+  if (M == 0) return 0;
+  if (M == 1) return one_map_identity(out_transforms);
+  int first, count;
+  block_of(R, W, M, &first, &count);
+  if ((int)local.size() != count) throw std::runtime_error("estimateMapsTransforms (multi-GPU): this rank's block holds " + std::to_string(count) + " maps");
+  Phases ph(c, phase_ms);
+
+  // ---- A: feature pipeline of the own block
+  std::vector<MapFeat> f;
+  compute_features(c, local, p, f, stage_ms);
+  const int dim = desc_dim(p);
+  ph.mark(0);
+
+  // ---- B, C: every map's sizes and features; a single rank has them all already
+  std::vector<int> npt(M), nkp(M);
+  std::vector<FeatView> views;
+  DBuf<float> all;
+  if (W > 1) {
+    views = exchange_features(c, cm, M, f, dim, all, npt, nkp);
+    f.clear();  // the views point into `all`
+  } else {
+    views = feat_views(f);
+    for (int m = 0; m < M; ++m) {
+      npt[m] = f[m].cloud.n;
+      nkp[m] = f[m].keypoints.n;
+    }
+  }
   ph.mark(1);
 
-  // ---- D: the row-major pair list (map_merging.cpp:246-254), dealt out by LPT — identical on every rank
-  std::vector<PairJob> pairs;
-  for (int i = 0; i < M - 1; ++i)
-    for (int j = i + 1; j < M; ++j)
-      if (nkp[i] > 0 && nkp[j] > 0) pairs.push_back(PairJob{i, j});
+  // ---- D: the row-major pair list, dealt out by LPT — identical on every rank
+  const std::vector<PairJob> pairs = row_major_pairs(nkp);
   const int P = (int)pairs.size();
-  std::vector<double> cost(P);
-  for (int k = 0; k < P; ++k) cost[k] = pair_cost(npt[pairs[k].a], npt[pairs[k].b], nkp[pairs[k].a], nkp[pairs[k].b], dim);
-  std::vector<int> owner;
-  lpt_assign(pairs, cost, W, owner);
+  const std::vector<int> owner = pair_owners(pairs, npt, nkp, dim, W);
   std::vector<PairJob> mine;
   std::vector<int> mine_k;
   for (int k = 0; k < P; ++k)
@@ -298,7 +333,7 @@ int dist_estimate(Ctx& c, mm3d_comm* cm, int n_maps, const std::vector<CloudView
 
   // ---- E: register the own share
   std::vector<PairOut> po;
-  register_pairs(c, views, dim, mine, p, po, nullptr);
+  register_pairs(c, views, dim, mine, p, po, stage_ms);
   ph.mark(2);
 
   // ---- F: results into their row-major slots
@@ -342,34 +377,22 @@ int dist_estimate(Ctx& c, mm3d_comm* cm, int n_maps, const std::vector<CloudView
   std::vector<std::vector<float>> g = compute_global_transforms(est, p.confidence_threshold, nullptr, nullptr, nullptr, nullptr);
   for (size_t i = 0; i < g.size(); ++i) to_colmajor(g[i].data(), out_transforms + 16 * i);
   ph.mark(4);
+  HostProf& hp = host_prof();
+  if (hp.on) {
+    fprintf(stderr, "[mm3d host] buffer allocations %ld calls %.2f ms (%.1f MB), cudaFreeAsync %ld calls %.2f ms, sync %ld calls %.2f ms, "
+            "small copies %ld calls %.2f ms; block cache holds %.1f MB\n", hp.n_alloc, hp.alloc_ms, hp.alloc_bytes / 1e6, hp.n_free, hp.free_ms,
+            hp.n_sync, hp.sync_ms, hp.n_copy, hp.copy_ms, c.cache->held_bytes / 1e6);
+    const bool on = hp.on;
+    hp = HostProf();
+    hp.on = on;
+  }
   return (int)g.size();
 }
 
-// Balanced key-range splitters from the all-reduced bucket histogram: splitters[r] <= bucket < splitters[r + 1] goes to rank r.
-std::vector<int> choose_splitters(const std::vector<unsigned long long>& hist, int world)
-{
-  const int nb = (int)hist.size();
-  std::vector<unsigned long long> cum(nb);
-  unsigned long long run = 0;
-  for (int i = 0; i < nb; ++i) { run += hist[i]; cum[i] = run; }
-  const unsigned long long total = run;
-  std::vector<int> sp(world + 1, 0);
-  sp[world] = nb;
-  for (int r = 1; r < world; ++r) {
-    const unsigned long long target = total * (unsigned long long)r / (unsigned long long)world;
-    int pos = (int)(std::lower_bound(cum.begin(), cum.end(), target) - cum.begin());
-    pos += total ? 1 : 0;
-    sp[r] = std::min(std::max(pos, sp[r - 1]), nb);
-  }
-  return sp;
-}
-
-}  // namespace
-
-namespace mm3d {
-
 // One rank's part of composeMaps: local clouds already on the device.  Returns this rank's slice of the composed map on the
 // host (host_out_alloc, records in out_layout); the slices concatenated in rank order are the reference's output bit for bit.
+// A single rank voxel-grids its concatenation as it is: voxel_downsample_batch applies pcl::VoxelGrid's overflow guard
+// itself, so the bounding box, key histogram and splitters are work of several ranks only.
 void dist_compose(Ctx& c, mm3d_comm* cm, const std::vector<CloudView>& local, const std::vector<const float*>& transforms_rowmajor,
                   double resolution, const mm3d_layout& out_layout, void** out, uint64_t* n_out)
 {
@@ -377,22 +400,36 @@ void dist_compose(Ctx& c, mm3d_comm* cm, const std::vector<CloudView>& local, co
   constexpr int NB = 4096;
   *out = nullptr;
   *n_out = 0;
-  // MM3D_HOST_TRACE=1: host wall clock between the phases (each ends in a synchronisation of its own)
+  // MM3D_HOST_TRACE=1: host wall clock between the phases (each ends in a synchronisation)
   const bool trace = host_prof().on;
-  double t_prev = trace ? now_ms() : 0.0;
+  double t_prev = trace ? host_now_ms() : 0.0;
   auto mark = [&](const char* what) {
     if (!trace) return;
-    const double t = now_ms();
+    c.sync();
+    const double t = host_now_ms();
     fprintf(stderr, "[mm3d compose] %s %.2f ms\n", what, t - t_prev);
     t_prev = t;
   };
+  auto to_host = [&](const float4* p, size_t n) {
+    *out = download_records(c, p, n, out_layout);
+    *n_out = n;
+    c.sync();
+    mark("copy to the host");
+  };
   DCloud cat;
   transform_concat(c, local, transforms_rowmajor, cat);
+  if (W == 1) {
+    std::vector<DCloud> res;
+    voxel_downsample_batch(c, {cat.view()}, (float)resolution, res, nullptr);
+    mark("transform + concatenate + voxel grid");
+    to_host(res[0].pts.p, (size_t)res[0].n);
+    return;
+  }
   float bbox[6];
   compose_bbox(c, cat, bbox);
   mark("transform + concatenate + bounding box");
   unsigned long long total = (unsigned long long)cat.n;
-  if (W > 1) {
+  {
     // min over ranks of (lo, -hi) and the point count
     float h[6] = {bbox[0], bbox[1], bbox[2], -bbox[3], -bbox[4], -bbox[5]};
     DBuf<float> d(c, 6);
@@ -408,12 +445,6 @@ void dist_compose(Ctx& c, mm3d_comm* cm, const std::vector<CloudView>& local, co
     c.sync();
     for (int k = 0; k < 3; ++k) { bbox[k] = h[k]; bbox[3 + k] = -h[3 + k]; }
   }
-  auto to_host = [&](const float4* p, size_t n) {
-    *out = download_records(c, p, n, out_layout);
-    *n_out = n;
-    c.sync();
-    mark("copy to the host");
-  };
   if (total == 0) {
     to_host(nullptr, 0);
     return;
@@ -421,14 +452,6 @@ void dist_compose(Ctx& c, mm3d_comm* cm, const std::vector<CloudView>& local, co
   const KeyGeomHost g = compose_geometry(bbox, resolution, NB);
   if (g.passthrough) {  // pcl::VoxelGrid's overflow guard: the composed map is the plain concatenation, rank order = map order
     to_host(cat.pts.p, (size_t)cat.n);
-    return;
-  }
-  if (W == 1) {
-    std::vector<DCloud> res;
-    voxel_downsample_batch(c, {cat.view()}, (float)resolution, res, nullptr);
-    if (trace) c.sync();
-    mark("voxel grid");
-    to_host(res[0].pts.p, (size_t)res[0].n);
     return;
   }
   std::vector<unsigned long long> hist(NB);
@@ -472,13 +495,47 @@ void dist_compose(Ctx& c, mm3d_comm* cm, const std::vector<CloudView>& local, co
 }
 
 // composeMaps' skip rules (map_merging.cpp:293-295): zero transforms and empty clouds are left out
-bool skip_map(const float* colmajor, const void* cloud, uint64_t n, float* rowmajor)
+bool skip_map(const float* colmajor, uint64_t n, float* rowmajor)
 {
   from_colmajor(colmajor, rowmajor);
   bool zero = true;  // Eigen isZero(): every |a_ij| <= 1e-5
   for (int k = 0; k < 16; ++k)
     if (!(std::fabs(rowmajor[k]) <= 1e-5f)) zero = false;
-  return zero || !cloud || n == 0;
+  return zero || n == 0;
+}
+
+KeptMaps kept_maps(const float* transforms_colmajor, const std::vector<uint64_t>& n_points)
+{
+  KeptMaps k;
+  for (int m = 0; m < (int)n_points.size(); ++m) {
+    float rm[16];
+    if (skip_map(transforms_colmajor + 16 * m, n_points[m], rm)) continue;
+    k.maps.push_back(m);
+    k.rowmajor.insert(k.rowmajor.end(), rm, rm + 16);
+  }
+  return k;
+}
+
+std::vector<const float*> KeptMaps::transforms() const
+{
+  std::vector<const float*> t(maps.size());
+  for (size_t i = 0; i < maps.size(); ++i) t[i] = rowmajor.data() + 16 * i;
+  return t;
+}
+
+std::vector<DCloud> upload_kept(Ctx& c, const void* const* clouds, const uint64_t* n_points, int first, int count, const float* transforms_colmajor,
+                                const mm3d_layout& l, KeptMaps& kept)
+{
+  std::vector<uint64_t> n(count);
+  for (int m = 0; m < count; ++m) n[m] = clouds[first + m] ? n_points[first + m] : 0;
+  kept = kept_maps(transforms_colmajor + 16 * first, n);
+  std::vector<const void*> src;
+  std::vector<uint64_t> cnt;
+  for (int m : kept.maps) {
+    src.push_back(clouds[first + m]);
+    cnt.push_back(n[m]);
+  }
+  return upload_clouds(c, src, cnt, l);
 }
 
 }  // namespace mm3d
@@ -539,9 +596,7 @@ int team_estimate(mm3d_ctx* master, int n_maps, const void* const* clouds, const
     block_of(r, W, n_maps, &first, &count);
     std::vector<DCloud> d = upload_clouds(c, std::vector<const void*>(clouds + first, clouds + first + count),
                                           std::vector<uint64_t>(n_points + first, n_points + first + count), layout);
-    std::vector<CloudView> v(count);
-    for (int m = 0; m < count; ++m) v[m] = d[m].view();
-    counts[r] = dist_estimate(c, cm, n_maps, v, p, outs[r].data(), nullptr);
+    counts[r] = dist_estimate(c, cm, n_maps, views(d), p, outs[r].data(), nullptr, nullptr);
     c.sync();
   });
   n_out = counts[0];
@@ -560,24 +615,9 @@ void team_compose(mm3d_ctx* master, int n_maps, const void* const* clouds, const
     team_run(master, [&](int r, Ctx& c, mm3d_comm* cm) {
       int first, count;
       block_of(r, W, n_maps, &first, &count);
-      std::vector<const void*> src;
-      std::vector<uint64_t> cnt;
-      std::vector<std::vector<float>> tr;
-      for (int m = first; m < first + count; ++m) {
-        float rm[16];
-        if (skip_map(transforms + 16 * m, clouds[m], n_points[m], rm)) continue;
-        src.push_back(clouds[m]);
-        cnt.push_back(n_points[m]);
-        tr.emplace_back(rm, rm + 16);
-      }
-      std::vector<DCloud> d = upload_clouds(c, src, cnt, in_layout);
-      std::vector<CloudView> v;
-      std::vector<const float*> tp;
-      for (size_t i = 0; i < d.size(); ++i) {
-        v.push_back(d[i].view());
-        tp.push_back(tr[i].data());
-      }
-      dist_compose(c, cm, v, tp, resolution, out_layout, &parts[r], &sizes[r]);
+      KeptMaps k;
+      std::vector<DCloud> d = upload_kept(c, clouds, n_points, first, count, transforms, in_layout, k);
+      dist_compose(c, cm, views(d), k.transforms(), resolution, out_layout, &parts[r], &sizes[r]);
     });
   } catch (...) {
     for (void* p : parts) host_out_free(p);
@@ -619,31 +659,11 @@ int mm3d_comm_id(void* id)
   return MM3D_OK;
 }
 
-#define MMD_TRY(ctx) \
-  if (!(ctx)) return MM3D_ERR_ARG; \
-  Ctx& c = (ctx)->c; \
-  try { \
-    MM_CUDA(cudaSetDevice(c.device));
-#define MMD_CATCH \
-  } catch (const UnsupportedError& e) { \
-    c.err = e.what(); \
-    return MM3D_ERR_UNSUPPORTED; \
-  } catch (const CudaError& e) { \
-    c.err = e.what(); \
-    cudaGetLastError(); \
-    return MM3D_ERR_CUDA; \
-  } catch (const std::exception& e) { \
-    c.err = e.what(); \
-    cudaGetLastError(); \
-    return MM3D_ERR; \
-  } \
-  return MM3D_OK;
-
 int mm3d_comm_create(mm3d_ctx* ctx, int rank, int world, const void* id, mm3d_comm** comm)
 {
   if (!comm || !id || world < 1 || rank < 0 || rank >= world) return MM3D_ERR_ARG;
   *comm = nullptr;
-  MMD_TRY(ctx)
+  MM_TRY(ctx)
   std::unique_ptr<mm3d_comm> h(new mm3d_comm);
   h->rank = rank;
   h->world = world;
@@ -651,7 +671,7 @@ int mm3d_comm_create(mm3d_ctx* ctx, int rank, int world, const void* id, mm3d_co
   memcpy(&u, id, sizeof(u));
   MM_NCCL(nccl().CommInitRank(&h->comm, world, u, rank));
   *comm = h.release();
-  MMD_CATCH
+  MM_CATCH
 }
 
 void mm3d_comm_destroy(mm3d_comm* comm)
@@ -675,21 +695,14 @@ int mm3d_dist_plan(int n_maps, const int32_t* n_points, const int32_t* n_keypoin
                    int* n_pairs)
 {
   if (n_maps < 0 || world < 1 || !n_points || !n_keypoints || !n_pairs) return MM3D_ERR_ARG;
-  std::vector<double> cost;
-  std::vector<PairJob> pj;
-  int P = 0;
-  for (int i = 0; i < n_maps - 1; ++i)
-    for (int j = i + 1; j < n_maps; ++j)
-      if (n_keypoints[i] > 0 && n_keypoints[j] > 0) {
-        if (pairs) { pairs[2 * P] = i; pairs[2 * P + 1] = j; }
-        pj.push_back(PairJob{i, j});
-        cost.push_back(pair_cost(n_points[i], n_points[j], n_keypoints[i], n_keypoints[j], dim));
-        ++P;
-      }
-  std::vector<int> own;
-  lpt_assign(pj, cost, world, own);
-  if (owner)
-    for (int k = 0; k < P; ++k) owner[k] = own[k];
+  const std::vector<int> npt(n_points, n_points + n_maps), nkp(n_keypoints, n_keypoints + n_maps);
+  const std::vector<PairJob> pj = row_major_pairs(nkp);
+  const std::vector<int> own = pair_owners(pj, npt, nkp, dim, world);
+  const int P = (int)pj.size();
+  for (int k = 0; k < P; ++k) {
+    if (pairs) { pairs[2 * k] = pj[k].a; pairs[2 * k + 1] = pj[k].b; }
+    if (owner) owner[k] = own[k];
+  }
   *n_pairs = P;
   return MM3D_OK;
 }
@@ -699,18 +712,14 @@ int mm3d_estimate_maps_transforms_dist(mm3d_ctx* ctx, mm3d_comm* comm, int n_map
 {
   if (!n_out || !params || n_maps < 0) return MM3D_ERR_ARG;
   *n_out = 0;
-  MMD_TRY(ctx)
+  MM_TRY(ctx)
   int first, count;
   block_of(comm ? comm->rank : 0, comm ? comm->world : 1, n_maps, &first, &count);
-  std::vector<DCloud> d(count);
-  std::vector<CloudView> v(count);
-  for (int m = 0; m < count; ++m) {
-    d[m] = upload_cloud(c, clouds[first + m], clouds[first + m] ? n_points[first + m] : 0);
-    v[m] = d[m].view();
-  }
-  *n_out = dist_estimate(c, comm, n_maps, v, *params, out_transforms, nullptr);
+  std::vector<DCloud> d = upload_clouds(c, std::vector<const void*>(clouds + first, clouds + first + count),
+                                        std::vector<uint64_t>(n_points + first, n_points + first + count), kPackedLayout);
+  *n_out = dist_estimate(c, comm, n_maps, views(d), *params, out_transforms, nullptr, nullptr);
   c.sync();
-  MMD_CATCH
+  MM_CATCH
 }
 
 int mm3d_estimate_resident_dist(mm3d_ctx* ctx, mm3d_comm* comm, int n_maps, const mm3d_maps* local_maps, const mm3d_params* params,
@@ -718,12 +727,10 @@ int mm3d_estimate_resident_dist(mm3d_ctx* ctx, mm3d_comm* comm, int n_maps, cons
 {
   if (!n_out || !params || !local_maps || n_maps < 0) return MM3D_ERR_ARG;
   *n_out = 0;
-  MMD_TRY(ctx)
-  std::vector<CloudView> v(local_maps->clouds.size());
-  for (size_t m = 0; m < v.size(); ++m) v[m] = local_maps->clouds[m].view();
-  *n_out = dist_estimate(c, comm, n_maps, v, *params, out_transforms, phase_ms);
+  MM_TRY(ctx)
+  *n_out = dist_estimate(c, comm, n_maps, views(local_maps->clouds), *params, out_transforms, phase_ms, nullptr);
   c.sync();
-  MMD_CATCH
+  MM_CATCH
 }
 
 int mm3d_compose_maps_dist(mm3d_ctx* ctx, mm3d_comm* comm, int n_local, const float* const* clouds, const uint64_t* n_points,
@@ -736,23 +743,11 @@ int mm3d_compose_maps_dist(mm3d_ctx* ctx, mm3d_comm* comm, int n_local, const fl
     if (ctx) ctx->c.err = "composeMaps: clouds and transforms size must be the same.";
     return MM3D_ERR_ARG;
   }
-  MMD_TRY(ctx)
-  std::vector<DCloud> d;
-  std::vector<std::vector<float>> tr;
-  for (int m = 0; m < n_local; ++m) {
-    float rm[16];
-    if (skip_map(transforms + 16 * m, clouds[m], n_points[m], rm)) continue;
-    d.push_back(upload_cloud(c, clouds[m], n_points[m]));
-    tr.emplace_back(rm, rm + 16);
-  }
-  std::vector<CloudView> v;
-  std::vector<const float*> tp;
-  for (size_t i = 0; i < d.size(); ++i) {
-    v.push_back(d[i].view());
-    tp.push_back(tr[i].data());
-  }
-  dist_compose(c, comm, v, tp, resolution, kPackedLayout, (void**)out, n_out);
-  MMD_CATCH
+  MM_TRY(ctx)
+  KeptMaps k;
+  std::vector<DCloud> d = upload_kept(c, (const void* const*)clouds, n_points, 0, n_local, transforms, kPackedLayout, k);
+  dist_compose(c, comm, views(d), k.transforms(), resolution, kPackedLayout, (void**)out, n_out);
+  MM_CATCH
 }
 
 int mm3d_compose_resident_dist(mm3d_ctx* ctx, mm3d_comm* comm, const mm3d_maps* local_maps, int n_transforms, const float* transforms,
@@ -765,20 +760,14 @@ int mm3d_compose_resident_dist(mm3d_ctx* ctx, mm3d_comm* comm, const mm3d_maps* 
     if (ctx) ctx->c.err = "composeMaps: clouds and transforms size must be the same.";
     return MM3D_ERR_ARG;
   }
-  MMD_TRY(ctx)
-  std::vector<std::vector<float>> tr;
+  MM_TRY(ctx)
+  std::vector<uint64_t> n;
+  for (const DCloud& d : local_maps->clouds) n.push_back((uint64_t)d.n);
+  const KeptMaps k = kept_maps(transforms, n);
   std::vector<CloudView> v;
-  std::vector<const float*> tp;
-  float dummy = 0.f;
-  for (int m = 0; m < n_transforms; ++m) {
-    float rm[16];
-    if (skip_map(transforms + 16 * m, &dummy, (uint64_t)local_maps->clouds[m].n, rm)) continue;
-    v.push_back(local_maps->clouds[m].view());
-    tr.emplace_back(rm, rm + 16);
-  }
-  for (size_t i = 0; i < tr.size(); ++i) tp.push_back(tr[i].data());
-  dist_compose(c, comm, v, tp, resolution, kPackedLayout, (void**)out, n_out);
-  MMD_CATCH
+  for (int m : k.maps) v.push_back(local_maps->clouds[m].view());
+  dist_compose(c, comm, v, k.transforms(), resolution, kPackedLayout, (void**)out, n_out);
+  MM_CATCH
 }
 
 int mm3d_create_multi(mm3d_ctx** ctx, const int* devices, int n_devices)

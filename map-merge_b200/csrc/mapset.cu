@@ -113,11 +113,7 @@ int mapset_estimate(Ctx& c, mm3d_mapset& s, const mm3d_params& p, float* out_tra
 {
   const int M = (int)s.slots.size();
   if (M == 0) return 0;
-  if (M == 1) {  // map_merging.cpp:192-197: no device work; the slot stays dirty
-    const float id[16] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1};
-    memcpy(out_transforms, id, sizeof(id));
-    return 1;
-  }
+  if (M == 1) return one_map_identity(out_transforms);  // no device work; the slot stays dirty
   check_supported(p);  // as compute_features does in the stateless call, even when nothing is left to compute
   const bool all = !s.have_params || !same_params(s.params, p);
   std::vector<char> dirty(M);
@@ -140,15 +136,13 @@ int mapset_estimate(Ctx& c, mm3d_mapset& s, const mm3d_params& p, float* out_tra
     for (size_t k = 0; k < computed.size(); ++k) fresh[computed[k]] = std::move(f[k]);
   }
   std::vector<FeatView> fv(M);
+  std::vector<int> nkp(M);
   for (int m = 0, t = 0; m < M; ++m) {
     const MapFeat& f = dirty[m] ? fresh[t++] : s.slots[m].feat;
     fv[m] = FeatView{f.cloud.view(), f.keypoints.view(), f.desc.p};
+    nkp[m] = f.keypoints.n;
   }
-  // src/map_merging.cpp:246-254
-  std::vector<PairJob> all_pairs;
-  for (int i = 0; i < M - 1; ++i)
-    for (int j = i + 1; j < M; ++j)
-      if (fv[i].keypoints.n > 0 && fv[j].keypoints.n > 0) all_pairs.push_back(PairJob{i, j});
+  const std::vector<PairJob> all_pairs = row_major_pairs(nkp);
   const int P = (int)all_pairs.size();
   // SAC_IA: where each pair's draws start.  Without a changed map no pair's features, and so no offset, can have moved.
   const bool walk = p.estimation_method == MM3D_EST_SAC_IA && !todo.empty();
@@ -303,18 +297,12 @@ int mm3d_mapset_compose(mm3d_ctx* ctx, const mm3d_mapset* set, int n_transforms,
   if (M != n_transforms) return arg_error(ctx, "composeMaps: clouds and transforms size must be the same.");
   if (!transforms) return arg_error(ctx, "mm3d_mapset_compose: transforms is NULL");
   MM_TRY(ctx)
-  std::vector<std::vector<float>> tr;
+  std::vector<uint64_t> n;
+  for (const Slot& sl : set->slots) n.push_back((uint64_t)sl.raw.n);
+  const KeptMaps k = kept_maps(transforms, n);
   std::vector<CloudView> v;
-  std::vector<const float*> tp;
-  const float any = 0.f;  // skip_map only tests the cloud pointer of host input for NULL
-  for (int m = 0; m < M; ++m) {
-    float rm[16];
-    if (skip_map(transforms + 16 * m, &any, (uint64_t)set->slots[m].raw.n, rm)) continue;
-    v.push_back(set->slots[m].raw.view());
-    tr.emplace_back(rm, rm + 16);
-  }
-  for (size_t i = 0; i < tr.size(); ++i) tp.push_back(tr[i].data());
-  dist_compose(c, nullptr, v, tp, resolution, *out_layout, out, n_out);
+  for (int m : k.maps) v.push_back(set->slots[m].raw.view());
+  dist_compose(c, nullptr, v, k.transforms(), resolution, *out_layout, out, n_out);
   MM_CATCH
 }
 
